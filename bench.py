@@ -2,6 +2,7 @@
 and the CPU baselines.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--envs-per-gpu E] [--legs a,b,...]
+                  [--dump-outputs DIR]
   torchrun --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 A "step" is one batched environment step of every env on every GPU: rs_step (move, obstruction collision, line of sight,
@@ -11,9 +12,9 @@ enforced boundaries, uniform random actions 0..7, episodes staggered so that ~1/
 Weak scaling: envs shard independently over ranks, no data-path collective.
 
 What the JSON line carries (rank 0 prints it):
-  value / ms_per_step   device-resident env-steps/s: the K-step window is run `reps` times, every window bracketed by a
-                        barrier + synchronize on both sides and timed with CUDA events, MAX over ranks per window, MEDIAN
-                        over the windows (min / max alongside)
+  value / ms_per_step   device-resident env-steps/s over exactly K timed steps: one window bracketed by a barrier +
+                        synchronize on both sides, its launches queued before its first kernel starts, timed with CUDA
+                        events, MAX over ranks
   roofline              the step kernel alone against the HBM roofline (algorithmic bytes SURVEY.md 8d)
   exact_poisson         the same headline with the numpy-exact PTRS sampler instead of the KS-equivalent fast one
   sweep                 BASELINE configs[1] (1,024 envs, 1-5 obstructions) and configs[2]'s size (65,536 envs): per-launch
@@ -27,6 +28,9 @@ What the JSON line carries (rank 0 prints it):
                         next to the measured ceiling of the device->host link
   cpu_baseline          the oracle's C port of the reference's per-env loop on the box's host cores (+ the reference's own
                         Python, timed in the build container, as secondary keys)
+
+The inputs are seeded and the number of steps before and inside the timed window depends on the arguments only, so
+`--dump-outputs DIR` (what the headline's last step handed its caller, see dump_outputs) can be compared between builds.
 """
 from __future__ import annotations
 
@@ -41,6 +45,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True                   # the benchmark runs from a built tree and leaves it as it found it
 
 METRIC = "RadSearch env-steps/sec (5 obstructions)"
 UNIT = "env-steps/s"
@@ -48,6 +53,9 @@ K_OBS = 5
 BYTES_PER_ENV_STEP = 122 + 32 * K_OBS        # SURVEY.md 8(d): algorithmic bytes per env-step, single agent
 GAE_BYTES_PER_ELEM = 17                      # SURVEY.md 8(d): rew 4 + val 4 + path_end 1 + adv 4 + ret 4
 T_EPOCH = 480
+PREROLL_STEPS = 20000                        # untimed steps before the timed window: ~0.6 s at 131,072 envs on a B200
+GATE_CYCLES = 1000000                        # device sleep the timed window's launches queue behind: ~0.5 ms
+DUMP_BYTES = 64 << 20                        # --dump-outputs writes at most this much
 ALL_LEGS = ("exact", "sweep", "gae", "pipeline", "maps", "e2e", "cpu")
 
 
@@ -258,11 +266,12 @@ def make_ring(cx: Ctx, N: int, R: int, fast: bool, episode_steps: int, graph: bo
     return envs
 
 
-def headline(cx: Ctx, envs, K: int, W: int, reps: int, sample_clocks: bool):
-    """Device-resident throughput of the ring of env batches: K steps per window, `reps` windows.  Batch r lives on its own
+def headline(cx: Ctx, envs, K: int, W: int, sample_clocks: bool):
+    """Device-resident throughput of the ring of env batches over one timed window of K steps.  Batch r lives on its own
     stream, so that the short tail kernels of one batch (reset of finished envs) and the drain of its step kernel's last
     CTAs overlap the next batch's step kernel.  Whole blocks of PREFETCH_PERIOD steps are one CUDA-graph launch
-    (RadSearch.step_block); a K that is not a multiple of the period runs step by step."""
+    (RadSearch.step_block); a K that is not a multiple of the period runs step by step.  How many steps run before the
+    timed window depends on K and W only, so the state the window leaves behind is the same from run to run."""
     torch = cx.torch
     R, N = len(envs), envs[0].num_envs
     P = envs[0].PREFETCH_PERIOD
@@ -290,37 +299,60 @@ def headline(cx: Ctx, envs, K: int, W: int, reps: int, sample_clocks: bool):
         for st in streams:
             main.wait_stream(st)
 
-    window(-(-max(W, 3) // P) * P)                       # warm-up: at least W steps, whole blocks
+    warm = -(-max(W, 3) // P) * P                        # warm-up: at least W steps, whole blocks
+    window(warm)
     cx.barrier()
     sampler = ClockSampler(cx.local_rank)
     if sample_clocks and cx.rank == 0:
         sampler.start()
-    # nvidia-smi samples every 100 ms: the same windows keep running (untimed) for 0.6 s in front of the timed ones so that
-    # the clock samples are taken under this very load
-    t_pre, pre = time.perf_counter(), 0
-    while time.perf_counter() - t_pre < 0.6:
+    # nvidia-smi samples every 100 ms: the same windows keep running (untimed) for PREROLL_STEPS steps in front of the timed
+    # one, so that the clocks have settled and their samples are taken under this very load.  A step count, not a time:
+    # the state at the end of the timed window must not depend on how fast the box ran.
+    pre = 0
+    while pre < PREROLL_STEPS:
         for _ in range(8):
             window(K)
             pre += K
         torch.cuda.synchronize()
-    times = []
-    for _ in range(reps):
-        cx.barrier()
-        e0, e1 = cx.event(), cx.event()
-        e0.record()
-        window(K)
-        e1.record()
-        cx.barrier()
-        times.append(e0.elapsed_time(e1))
+    cx.barrier()
+    # the window's launches queue up behind a short sleep on the main stream, so that its time is the GPU's for K steps
+    # and not the host's launch latency after the barrier (~30 us on a B200, 5 % of a 20-step window at 131,072 envs)
+    torch.cuda._sleep(GATE_CYCLES)
+    e0, e1 = cx.event(), cx.event()
+    e0.record()
+    window(K)
+    e1.record()
+    cx.barrier()
     clocks = sampler.stop() if (sample_clocks and cx.rank == 0) else None
-    times = cx.max_over_ranks(times)
-    med = median(times)
+    ms = cx.max_over_ranks([e0.elapsed_time(e1)])[0]
     launches_per_step = (2 + 1.0 / P)
-    return {"ms": med, "ms_min": min(times), "ms_max": max(times), "reps": reps, "preroll_steps": pre,
-            "value": N * cx.world * K / (med / 1e3), "clocks": clocks, "launches": int(launches_per_step * K),
+    return {"ms": ms, "warmup_steps": warm, "preroll_steps": pre,
+            "value": N * cx.world * K / (ms / 1e3), "clocks": clocks, "launches": int(launches_per_step * K),
             "graph_launches": (K // P) if use_blocks else K,
             "mode": (f"one CUDA-graph launch per block of {P} steps" if use_blocks else "one CUDA-graph launch per step")
             if envs[0].use_cuda_graph else "stream launches"}
+
+
+def dump_outputs(cx: Ctx, envs, out_dir: str):
+    """Write what the headline's last step handed its caller: the six step outputs (obs, reward, team_reward, done_flags,
+    info_flags, ended) of every env batch of the ring, each as DIR/<name>.npy in float32 with the batches concatenated
+    along the env axis (row b * N + n = env n of batch b).  Above DUMP_BYTES in all, every array keeps the same fixed,
+    seeded sample of rows, whose row numbers go to DIR/env_index.npy (float64)."""
+    import numpy as np
+
+    torch = cx.torch
+    names = ("obs", "reward", "team_reward", "done_flags", "info_flags", "ended")
+    arrays = {n: torch.cat([getattr(e, n) for e in envs]).float() for n in names}
+    rows = len(envs) * envs[0].num_envs
+    row_bytes = sum(a[0].numel() * 4 for a in arrays.values())
+    budget = DUMP_BYTES - (64 << 10)                     # room for the .npy headers
+    os.makedirs(out_dir, exist_ok=True)
+    if rows * row_bytes > budget:
+        idx = torch.randperm(rows, generator=torch.Generator().manual_seed(0))[:budget // (row_bytes + 8)].sort().values
+        np.save(os.path.join(out_dir, "env_index.npy"), idx.double().numpy())
+        arrays = {n: a[idx.to(a.device)] for n, a in arrays.items()}
+    for n, a in arrays.items():
+        np.save(os.path.join(out_dir, n + ".npy"), a.cpu().numpy())
 
 
 def step_kernel_time(cx: Ctx, envs, groups: int, fast: bool):
@@ -891,7 +923,6 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--envs-per-gpu", type=int, default=131072)
     ap.add_argument("--ring", type=int, default=4, help="env batches cycled so that each step's state comes from HBM")
-    ap.add_argument("--reps", type=int, default=0, help="timed windows (0: 50, fewer for long windows)")
     ap.add_argument("--exact-poisson", action="store_true", help="fp64 numpy-exact PTRS acceptance as the headline sampler")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--quick", action="store_true", help="headline + step-kernel timing only (what the ncu passes replay)")
@@ -901,6 +932,7 @@ def main():
     ap.add_argument("--episode-steps", type=int, default=120, help="steps_per_episode (120 = the reference's; a huge value "
                     "shows the throughput without resets)")
     ap.add_argument("--period", type=int, default=0, help="steps per prefetch block / graph launch (0 = pick_period(steps))")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write rank 0's step outputs of the last timed step to DIR/*.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -912,12 +944,13 @@ def main():
     torch = cx.torch
     N, K, W, R = args.envs_per_gpu, args.steps, max(args.warmup, 3), max(args.ring, 1)
     fast = not args.exact_poisson
-    reps = args.reps if args.reps > 0 else max(10, min(50, int(2.0e6 / max(K * 20, 1))))
     graph, prefetch = not (args.no_graph or args.no_prefetch), not args.no_prefetch
 
     period = args.period or pick_period(K, args.episode_steps)
     envs = make_ring(cx, N, R, fast, args.episode_steps, graph, prefetch, period)
-    head = headline(cx, envs, K, W, reps, sample_clocks=True)
+    head = headline(cx, envs, K, W, sample_clocks=True)
+    if args.dump_outputs and cx.rank == 0:
+        dump_outputs(cx, envs, args.dump_outputs)
     k_mean, k_med, k_single, k_conc = step_kernel_time(cx, envs, 120, fast)
     achieved = BYTES_PER_ENV_STEP * N / (k_mean / 1e3) / 1e9
     state_mb = R * N * (BYTES_PER_ENV_STEP + 160 + 80 + 80) / 1e6
@@ -936,9 +969,10 @@ def main():
         "metric": METRIC, "value": head["value"], "unit": UNIT, "n_gpus": cx.world, "steps": K, "warmup": W,
         "ms_per_step": head["ms"] / K, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
         "dtype": "int32+f64", "data": "synthetic",
-        "timing": {"reps": head["reps"], "window_ms_median": head["ms"], "window_ms_min": head["ms_min"],
-                   "window_ms_max": head["ms_max"], "preroll_steps": head["preroll_steps"],
-                   "rule": "every K-step window bracketed by barrier + synchronize, CUDA events, max over ranks, median over windows"},
+        "timing": {"timed_steps": K, "window_ms": head["ms"], "warmup_steps": head["warmup_steps"],
+                   "preroll_steps": head["preroll_steps"],
+                   "rule": "one K-step window after the warm-up and pre-roll steps, bracketed by barrier + synchronize, "
+                           "launches queued behind a device sleep before the start event, CUDA events, max over ranks"},
         "config": {"workload": f"RadSearch env step + auto-reset, {N} envs/GPU (BASELINE configs[4]), 5 obstructions, "
                                f"enforced boundaries, 1 agent, uniform random actions, staggered {args.episode_steps}-step episodes",
                    "envs_per_gpu": N, "obstructions": K_OBS,
@@ -971,7 +1005,7 @@ def main():
         for e in envs:
             e._quiesce_prefetch()
         envs_x = make_ring(cx, N, 2, False, args.episode_steps, graph, prefetch)
-        hx = headline(cx, envs_x, K, W, max(10, reps // 2), sample_clocks=False)
+        hx = headline(cx, envs_x, K, W, sample_clocks=False)
         kx_mean, _, kx_single, _ = step_kernel_time(cx, envs_x, 40, False)
         line["exact_poisson"] = {"value": hx["value"], "ms_per_step": hx["ms"] / K, "kernel_ms": kx_mean,
                                  "frac": BYTES_PER_ENV_STEP * N / (kx_mean / 1e3) / 1e9 / cx.peak,
