@@ -222,6 +222,23 @@ int rs_rollout_post(const float *reward, const uint8_t *ended, const uint8_t *do
                     float *boot_row, float *hidden, int32_t hidden_dim, double *ep_return, int32_t *ep_steps, double *acc,
                     double *ep_min, double *ep_max, float *rew_row, uint8_t *end_row, int32_t n, int32_t last_step,
                     void *stream);
+/* The same two launches for n_agents (1..8) agents per environment (RAD-TEAM, T:321-571 multi-agent branch).  Columns are
+ * env-major, column n*A + a, the memory order of rs_step's [N][A] outputs.
+ * rs_rollout_pre_team: act_row / val_row / logp_row [N*A] <- action / val / logp [N][A]; pred_row [N*A][2] <- pred [N][A][2]
+ * (the PFGRU's source prediction; NULL pred writes NaN = none; pred_row nullable); src_row [N*A][2] <- src[n] broadcast to
+ * the env's A columns (nullable); obs_row [N*A][obs_dim] <- obs as in rs_rollout_pre (nullable).
+ * rs_rollout_post_team: rew_row[n*A + a] = individual ? reward[n][a] : team_reward[n] (T:361-375; nullable);
+ * end_row[n*A + a] = ended[n] (nullable); boot_row[n*A + a] = v_next[n][a] where the trajectory was cut, else 0;
+ * hidden [N*A][hidden_dim] restarted where ended[n] != 0 and not last_step; episode statistics (nullable as a group) with
+ * ep_return [N][A] f64 (returns of the same reward rule), ep_steps [N], acc [6][A], ep_min / ep_max [A]. */
+int rs_rollout_pre_team(const int32_t *action, const float *val, const float *logp, const float *pred, const int32_t *src,
+                        float *act_row, float *val_row, float *logp_row, float *pred_row, float *src_row, const float *obs,
+                        float *obs_row, int32_t obs_dim, int32_t n_env, int32_t n_agents, void *stream);
+int rs_rollout_post_team(const float *reward, const float *team_reward, const uint8_t *ended, const uint8_t *done,
+                         const uint8_t *info, const float *v_next, float *boot_row, float *hidden, int32_t hidden_dim,
+                         double *ep_return, int32_t *ep_steps, double *acc, double *ep_min, double *ep_max, float *rew_row,
+                         uint8_t *end_row, int32_t n_env, int32_t n_agents, int32_t individual, int32_t last_step,
+                         void *stream);
 
 /* ---- RAD-TEAM map observation (SURVEY.md 8f-1) ---------------------------------------------------------------------
  * MapsBuffer.observation_to_map (algos/multiagent/NeuralNetworkCores/RADTEAM_core.py:532-616 with its helpers :101-182
@@ -269,6 +286,20 @@ int rs_maps_update(const RsMapsConfig *cfg, const RsMapsState *st, const float *
 /* MapsBuffer.reset for the selected environments (mask NULL = all). */
 int rs_maps_reset(const RsMapsConfig *cfg, const RsMapsState *st, const uint8_t *mask, int32_t mask_bits, int32_t n_env,
                   void *stream);
+/* Map stacks for the PPO update, rebuilt from a rollout buffer instead of stored (one step's stacks are 4*(6A+4)*X*Y
+ * bytes per env; the inputs of the calls that made them are 52*A).  For each range i = (n, t0, t1) of ranges[m][3]
+ * (device), rows out_row0[i] .. out_row0[i] + t1 - t0 of out_actor [R][A][X][Y][6] / out_critic [R][X][Y][4] receive the
+ * stacks rs_maps_update had produced when the policy read env n's observation of step t = t0..t1: the calls on
+ * obs_rows[s..t] with pred_rows[s..t], s = 1 + the last path end before t in column n*A of end_rows (or 0).  A range
+ * may cross path ends; the replay restarts there.  obs_rows [T+1][N][A][11] (row t = what the policy saw at step t),
+ * pred_rows [T][N][A][2] (NaN = none; NULL = no predictions), end_rows [T][N*A] (the rollout buffer's path-end bytes).
+ * st: only visit_lut is read; nothing of the live state is read or written.  out_status[i] = the RS_MS_* bits of the
+ * replayed calls | RS_MR_BAD_RANGE when n is outside [0, N) or t0..t1 leaves [0, T) (its rows are zeroed) or t1 < t0
+ * (it owns no rows). */
+#define RS_MR_BAD_RANGE 8u
+int rs_maps_replay(const RsMapsConfig *cfg, const RsMapsState *st, const float *obs_rows, const float *pred_rows,
+                   const uint8_t *end_rows, int32_t T, int32_t n_env, const int32_t *ranges, int32_t m,
+                   const int64_t *out_row0, float *out_actor, float *out_critic, uint32_t *out_status, void *stream);
 int rs_sizeof_maps_config(void);
 int rs_sizeof_maps_state(void);
 

@@ -10,10 +10,11 @@ from .envs.rad_search_env import HostStepBuffers, RadSearch, StepResult
 from .ppo_buffer import (BatchedPPOBuffer, PPOBuffer, advantage_statistics, combined_shape, gae_advantages,
                          normalize_advantages_)
 from .dist import shard_range
-from .maps_buffer import BatchedMapsBuffer, MapsBuffer
+from .maps_buffer import BatchedMapsBuffer, MapsBuffer, episode_ranges
 from .evaluate import MonteCarloEvaluator, MonteCarloResults, uniform_policy
 from .rollout_stats import EpisodeStats
-from .rollout import RolloutCollector
+from .rollout import RolloutCollector, TeamRolloutCollector, TeamRolloutPolicy
 
 __all__ = ["RadSearch", "StepResult", "HostStepBuffers", "PPOBuffer", "BatchedPPOBuffer", "gae_advantages", "advantage_statistics",
-           "normalize_advantages_", "combined_shape", "shard_range", "BatchedMapsBuffer", "MapsBuffer", "MonteCarloEvaluator", "MonteCarloResults", "uniform_policy", "EpisodeStats", "RolloutCollector", "RadSearchLibraryError", "_lib"]
+           "normalize_advantages_", "combined_shape", "shard_range", "BatchedMapsBuffer", "MapsBuffer", "MonteCarloEvaluator", "MonteCarloResults", "uniform_policy", "EpisodeStats", "RolloutCollector",
+           "TeamRolloutCollector", "TeamRolloutPolicy", "episode_ranges", "RadSearchLibraryError", "_lib"]

@@ -40,45 +40,35 @@ __device__ __forceinline__ int cell_of(const RsMapsConfig &c, double vx, double 
     return cx * c.dim_y + cy;
 }
 
-__global__ void __launch_bounds__(kBlock) maps_update_kernel(const __grid_constant__ RsMapsConfig c,
-                                                             const __grid_constant__ RsMapsState S, const float *obs,
-                                                             const float *loc_pred, const uint8_t *mask, int mask_bits,
-                                                             int n_env) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    const int n = blockIdx.x * kWarpsPerBlock + w;
-    if (n >= n_env || (mask && !(mask[n] & mask_bits))) return;            // whole warps leave together
-    // per warp: the episode's sample table (values, cells) and the compaction scratch
-    float *s_val = reinterpret_cast<float *>(smem_raw) + (size_t)w * 2 * c.log_cap;
-    float *scratch = s_val + c.log_cap;
-    uint16_t *s_cell = reinterpret_cast<uint16_t *>(reinterpret_cast<float *>(smem_raw) + (size_t)kWarpsPerBlock * 2 * c.log_cap) +
-                       (size_t)w * c.log_cap;
+// The per-environment state of the map observation between two calls.  maps_update_kernel keeps it in HBM (RsMapsState)
+// and holds it here for the duration of a call; maps_replay_kernel keeps it here (and the sample table in shared memory)
+// for a whole replayed episode.  rec / last_pred are per lane (lane b: agent b); the rest is the same on every lane.
+struct MapsCallState {
+    int len;                 // readings in the sample table
+    double mean, m2;         // tools.standardizer
+    int cnt;
+    int rec, last_pred;      // tools.last_coords[b] / buffer b's last prediction cell (-1 = none)
+};
+
+// One observation_to_map call of environment n for all its A buffers (M:532-616), by one warp.  obs: the env's [A][11]
+// row; loc_pred: its [A][2] row or NULL; s_cell / s_val: the sample table staged in shared memory (st.len entries), and
+// log_cell / log_val its copy in HBM (NULL: none); scratch: log_cap floats of shared memory; actor: the env's [A][X][Y][6]
+// stacks, critic its [X][Y][4] stack.  The call only STORES into the stacks.  Returns the RS_MS_* bits of this lane.
+__device__ __forceinline__ uint32_t maps_call(const RsMapsConfig &c, const float *__restrict__ visit_lut, const float *obs,
+                                              const float *loc_pred, uint16_t *log_cell, float *log_val, uint16_t *s_cell,
+                                              float *s_val, float *scratch, float *actor_env, float *critic, int lane,
+                                              MapsCallState &st) {
     const int A = c.n_agents, XY = c.dim_x * c.dim_y;
     uint32_t status = 0;
-
-    // ---- everything the call reads from HBM is requested up front (one round of latency) ------------------------------
-    uint16_t *log_cell = S.log_cell + (size_t)n * c.log_cap;
-    float *log_val = S.log_val + (size_t)n * c.log_cap;
-    int len = S.log_len[n];
-    double mean = S.std[2 * (size_t)n], m2 = S.std[2 * (size_t)n + 1];
-    int cnt = S.std_count[n];
-    int rec = -1, last_pred = -1;                                           // lane b: tools.last_coords[b] / buffer b's last prediction
-    if (lane < A) {
-        rec = S.last_cell[(size_t)n * A + lane];
-        last_pred = S.last_pred[(size_t)n * A + lane];
-    }
-#pragma unroll 4
-    for (int i = lane; i < len; i += 32) {
-        s_cell[i] = log_cell[i];
-        s_val[i] = log_val[i];
-    }
+    int len = st.len, cnt = st.cnt, rec = st.rec;
+    double mean = st.mean, m2 = st.m2;
 
     // ---- this call's observations: lane a holds agent a -----------------------------------------------------------
     int my_cell = -1, my_pred = -1;
     float my_count = 0.0f, my_obst = 0.0f;
     bool my_has_obst = false, pred_given = false;
     if (lane < A) {
-        const float *o = obs + ((size_t)n * A + lane) * RS_OBS_DIM;
+        const float *o = obs + (size_t)lane * RS_OBS_DIM;
         my_count = o[0];
         // the env writes x * scale rounded to fp32; the reference's float64 observation is recovered from the lattice
         // coordinate (exact: the fp32 error is 1e-4 of a lattice step)
@@ -91,7 +81,7 @@ __global__ void __launch_bounds__(kBlock) maps_update_kernel(const __grid_consta
             if (v != 0.0f) { my_obst = v; my_has_obst = true; }
         }
         if (c.use_prediction && loc_pred) {
-            const float px = loc_pred[((size_t)n * A + lane) * 2], py = loc_pred[((size_t)n * A + lane) * 2 + 1];
+            const float px = loc_pred[(size_t)lane * 2], py = loc_pred[(size_t)lane * 2 + 1];
             if (px == px && py == py) {                                    // NaN = no prediction for this buffer
                 pred_given = true;
                 my_pred = cell_of(c, (double)px, (double)py);
@@ -104,8 +94,10 @@ __global__ void __launch_bounds__(kBlock) maps_update_kernel(const __grid_consta
     if (len + A <= c.log_cap) {
         if (lane < A) {
             const uint16_t cell16 = (uint16_t)(my_cell < 0 ? 0xffff : my_cell);
-            log_cell[len + lane] = cell16;
-            log_val[len + lane] = my_count;
+            if (log_cell) {
+                log_cell[len + lane] = cell16;
+                log_val[len + lane] = my_count;
+            }
             s_cell[len + lane] = cell16;
             s_val[len + lane] = my_count;
         }
@@ -117,16 +109,15 @@ __global__ void __launch_bounds__(kBlock) maps_update_kernel(const __grid_consta
 
     // stacks are stored cell-major, channel innermost ([X][Y][6] / [X][Y][4]): the values one call writes for a cell of
     // a buffer share a 32-byte sector or two instead of one sector per channel plane
-    float *actor = S.actor + ((size_t)n * A + (lane < A ? lane : 0)) * 6 * XY;   // lane a' owns buffer a'
-    float *critic = S.critic + (size_t)n * 4 * XY;
+    float *actor = actor_env + (size_t)(lane < A ? lane : 0) * 6 * XY;   // lane a' owns buffer a'
 #define ACT(ch, cell) actor[(size_t)(cell) * 6 + (ch)]
 #define CRI(ch, cell) critic[(size_t)(cell) * 4 + (ch)]
 
     // ---- source prediction map of buffer a' (PFGRU) M:564-568, 748-766: the old mark (a 1) goes, the new one is set ------
     if (pred_given) {
-        if (last_pred >= 0 && last_pred != my_pred) ACT(0, last_pred) = 0.0f;
+        if (st.last_pred >= 0 && st.last_pred != my_pred) ACT(0, st.last_pred) = 0.0f;
         if (my_pred >= 0) ACT(0, my_pred) = 1.0f;      // outside the map (the reference raises): old mark cleared, none set
-        S.last_pred[(size_t)n * A + lane] = my_pred;
+        st.last_pred = my_pred;
     }
 
     // ---- agents in dict order M:547-604 ---------------------------------------------------------------------------------
@@ -193,7 +184,7 @@ __global__ void __launch_bounds__(kBlock) maps_update_kernel(const __grid_consta
         // visit counts M:886-916: the shadow counter (2 per earlier visit of the cell) equals twice the number of the cell's
         // samples recorded before this agent's turn: all of them minus this call's readings of agents a..A-1 there
         const int later = __popc(__ballot_sync(0xffffffffu, lane < A && lane >= a && my_cell == cc));
-        const float vis = S.visit_lut[max(m - later, 0)];
+        const float vis = visit_lut[max(m - later, 0)];
 
         // agents recorded at the old / new cell after this move
         const int n_cc = __popc(__ballot_sync(0xffffffffu, lane < A && rec == cc));
@@ -220,16 +211,164 @@ __global__ void __launch_bounds__(kBlock) maps_update_kernel(const __grid_consta
     }
 #undef ACT
 #undef CRI
-    if (lane < A) S.last_cell[(size_t)n * A + lane] = rec;
+    st.len = len;
+    st.cnt = cnt;
+    st.rec = rec;
+    st.mean = mean;
+    st.m2 = m2;
+    return status;
+}
+
+__global__ void __launch_bounds__(kBlock) maps_update_kernel(const __grid_constant__ RsMapsConfig c,
+                                                             const __grid_constant__ RsMapsState S, const float *obs,
+                                                             const float *loc_pred, const uint8_t *mask, int mask_bits,
+                                                             int n_env) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const int n = blockIdx.x * kWarpsPerBlock + w;
+    if (n >= n_env || (mask && !(mask[n] & mask_bits))) return;            // whole warps leave together
+    // per warp: the episode's sample table (values, cells) and the compaction scratch
+    float *s_val = reinterpret_cast<float *>(smem_raw) + (size_t)w * 2 * c.log_cap;
+    float *scratch = s_val + c.log_cap;
+    uint16_t *s_cell = reinterpret_cast<uint16_t *>(reinterpret_cast<float *>(smem_raw) + (size_t)kWarpsPerBlock * 2 * c.log_cap) +
+                       (size_t)w * c.log_cap;
+    const int A = c.n_agents, XY = c.dim_x * c.dim_y;
+
+    // ---- everything the call reads from HBM is requested up front (one round of latency) ------------------------------
+    uint16_t *log_cell = S.log_cell + (size_t)n * c.log_cap;
+    float *log_val = S.log_val + (size_t)n * c.log_cap;
+    MapsCallState st;
+    st.len = S.log_len[n];
+    st.mean = S.std[2 * (size_t)n];
+    st.m2 = S.std[2 * (size_t)n + 1];
+    st.cnt = S.std_count[n];
+    st.rec = -1;
+    st.last_pred = -1;
+    if (lane < A) {
+        st.rec = S.last_cell[(size_t)n * A + lane];
+        st.last_pred = S.last_pred[(size_t)n * A + lane];
+    }
+    const int last_pred0 = st.last_pred;
+#pragma unroll 4
+    for (int i = lane; i < st.len; i += 32) {
+        s_cell[i] = log_cell[i];
+        s_val[i] = log_val[i];
+    }
+
+    uint32_t status = maps_call(c, S.visit_lut, obs + (size_t)n * A * RS_OBS_DIM,
+                                loc_pred ? loc_pred + (size_t)n * A * 2 : nullptr, log_cell, log_val, s_cell, s_val, scratch,
+                                S.actor + (size_t)n * A * 6 * XY, S.critic + (size_t)n * 4 * XY, lane, st);
+    if (lane < A) {
+        S.last_cell[(size_t)n * A + lane] = st.rec;
+        if (st.last_pred != last_pred0) S.last_pred[(size_t)n * A + lane] = st.last_pred;
+    }
     if (lane == 0) {
-        S.log_len[n] = len;
-        S.std[2 * (size_t)n] = mean;
-        S.std[2 * (size_t)n + 1] = m2;
-        S.std_count[n] = cnt;
+        S.log_len[n] = st.len;
+        S.std[2 * (size_t)n] = st.mean;
+        S.std[2 * (size_t)n + 1] = st.m2;
+        S.std_count[n] = st.cnt;
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) status |= __shfl_xor_sync(0xffffffffu, status, o);
     if (lane == 0 && status) S.status[n] |= status;
+}
+
+// Dense copy / zeroing of one output row of the replay (16-byte accesses when the row allows them).  A copy issues 8
+// loads per lane before their stores: one warp moves a whole row, so the loads in flight are what sets its rate.
+__device__ __forceinline__ void row_fill(float *dst, const float *src, size_t cnt, int lane) {
+    if ((cnt & 3) == 0 && (reinterpret_cast<uintptr_t>(dst) & 15) == 0 && (!src || (reinterpret_cast<uintptr_t>(src) & 15) == 0)) {
+        float4 *d4 = reinterpret_cast<float4 *>(dst);
+        const float4 *s4 = reinterpret_cast<const float4 *>(src);
+        const size_t n4 = cnt / 4;
+        if (!src) {
+            const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll 4
+            for (size_t i = lane; i < n4; i += 32) d4[i] = z4;
+            return;
+        }
+        size_t i = lane;
+        for (; i + 7 * 32 < n4; i += 8 * 32) {
+            float4 v[8];
+#pragma unroll
+            for (int k = 0; k < 8; k++) v[k] = s4[i + k * 32];
+#pragma unroll
+            for (int k = 0; k < 8; k++) d4[i + k * 32] = v[k];
+        }
+        for (; i < n4; i += 32) d4[i] = s4[i];
+    } else {
+        for (size_t i = lane; i < cnt; i += 32) dst[i] = src ? src[i] : 0.0f;
+    }
+}
+
+// The map stacks the policy read at steps t0..t1 of env n, rebuilt from the rollout buffer: one warp per requested range.
+// The first row is built by replaying the calls of rows s..t0 (s: the first row of t0's episode) into the zeroed output row;
+// every following row is the previous output row (dense copy) plus the sparse stores of its own call, or a zeroed row and
+// a restarted state where an episode starts inside the range.  The sample table lives in shared memory, the rest of the
+// state in registers: nothing of the live RsMapsState but the visit-count table is read.
+__global__ void __launch_bounds__(kBlock) maps_replay_kernel(const __grid_constant__ RsMapsConfig c, const float *visit_lut,
+                                                             const float *obs_rows, const float *pred_rows,
+                                                             const uint8_t *end_rows, int T, int n_env, const int32_t *ranges,
+                                                             int m, const int64_t *out_row0, float *out_actor,
+                                                             float *out_critic, uint32_t *out_status) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const int r = blockIdx.x * kWarpsPerBlock + w;
+    if (r >= m) return;
+    float *s_val = reinterpret_cast<float *>(smem_raw) + (size_t)w * 2 * c.log_cap;
+    float *scratch = s_val + c.log_cap;
+    uint16_t *s_cell = reinterpret_cast<uint16_t *>(reinterpret_cast<float *>(smem_raw) + (size_t)kWarpsPerBlock * 2 * c.log_cap) +
+                       (size_t)w * c.log_cap;
+    const int A = c.n_agents, XY = c.dim_x * c.dim_y, NA = n_env * A;
+    const size_t actor_row = (size_t)A * 6 * XY, critic_row = (size_t)4 * XY;
+    const int n = ranges[3 * (size_t)r], t0 = ranges[3 * (size_t)r + 1], t1 = ranges[3 * (size_t)r + 2];
+    const int64_t row0 = out_row0[r];
+    if (t1 < t0) {                                                          // inverted: owns no rows
+        if (lane == 0) out_status[r] = RS_MR_BAD_RANGE;
+        return;
+    }
+    if (n < 0 || n >= n_env || t0 < 0 || t1 >= T) {                         // outside the buffer: zero rows
+        for (int64_t k = 0; k <= (int64_t)t1 - t0; k++) {
+            row_fill(out_actor + (size_t)(row0 + k) * actor_row, nullptr, actor_row, lane);
+            row_fill(out_critic + (size_t)(row0 + k) * critic_row, nullptr, critic_row, lane);
+        }
+        if (lane == 0) out_status[r] = RS_MR_BAD_RANGE;
+        return;
+    }
+    // s: 1 + the last path end before t0 in column n*A (all agents of an env end together), or 0
+    int s = 0;
+    for (int hi = t0 - 1; hi >= 0; hi -= 32) {
+        const int t = hi - lane;
+        const bool e = t >= 0 && end_rows[(size_t)t * NA + (size_t)n * A] != 0;
+        const unsigned b = __ballot_sync(0xffffffffu, e);
+        if (b) { s = hi - (__ffs(b) - 1) + 1; break; }                      // lowest lane = latest row
+    }
+    uint32_t status = 0;
+    MapsCallState st;
+    float *act = out_actor + (size_t)row0 * actor_row, *cri = out_critic + (size_t)row0 * critic_row;
+    for (int t = s; t <= t1; t++) {
+        if (t == s || (t > t0 && end_rows[(size_t)(t - 1) * NA + (size_t)n * A] != 0)) {   // an episode starts: reset
+            if (t > t0) {
+                act += actor_row;
+                cri += critic_row;
+            }
+            row_fill(act, nullptr, actor_row, lane);
+            row_fill(cri, nullptr, critic_row, lane);
+            st.len = 0; st.mean = 0.0; st.m2 = 0.0; st.cnt = 0; st.rec = -1; st.last_pred = -1;
+        } else if (t > t0) {                                                // the next row starts as a copy of this one
+            row_fill(act + actor_row, act, actor_row, lane);
+            row_fill(cri + critic_row, cri, critic_row, lane);
+            act += actor_row;
+            cri += critic_row;
+        }
+        __syncwarp();
+        status |= maps_call(c, visit_lut, obs_rows + ((size_t)t * NA + (size_t)n * A) * RS_OBS_DIM,
+                            pred_rows ? pred_rows + ((size_t)t * NA + (size_t)n * A) * 2 : nullptr, nullptr, nullptr, s_cell,
+                            s_val, scratch, act, cri, lane, st);
+        __syncwarp();
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) status |= __shfl_xor_sync(0xffffffffu, status, o);
+    if (lane == 0) out_status[r] = status;
 }
 
 // MapsBuffer.reset M:513-523 (+ ConversionTools.reset M:378-385) for the selected environments: one warp zeroes the
@@ -307,6 +446,32 @@ int rs_maps_reset(const RsMapsConfig *cfg, const RsMapsState *st, const uint8_t 
     const int grid = (n_env + kWarpsPerBlock - 1) / kWarpsPerBlock;
     maps_reset_kernel<<<grid, kBlock, 0, static_cast<cudaStream_t>(stream)>>>(*cfg, *st, mask, mask_bits ? mask_bits : 0xff,
                                                                               n_env);
+    return (int)cudaGetLastError();
+}
+
+int rs_maps_replay(const RsMapsConfig *cfg, const RsMapsState *st, const float *obs_rows, const float *pred_rows,
+                   const uint8_t *end_rows, int32_t T, int32_t n_env, const int32_t *ranges, int32_t m,
+                   const int64_t *out_row0, float *out_actor, float *out_critic, uint32_t *out_status, void *stream) {
+    if (!cfg || !st) return rs_set_error("rs_maps_replay: maps cfg/state is NULL");
+    if (n_env <= 0 || T <= 0) return rs_set_error("rs_maps_replay: T and n_env must be positive");
+    if (m < 0) return rs_set_error("rs_maps_replay: m must be >= 0");
+    if (cfg->n_agents < 1 || cfg->n_agents > RS_MAX_A) return rs_set_error("rs_maps_replay: n_agents out of range [1, 8]");
+    if (cfg->dim_x < 1 || cfg->dim_y < 1 || (int64_t)cfg->dim_x * cfg->dim_y > 65535)
+        return rs_set_error("rs_maps_replay: map dimensions out of range");
+    if (cfg->log_cap < cfg->n_agents || cfg->log_cap > 8192) return rs_set_error("rs_maps_replay: log_cap out of range");
+    if (!(cfg->resolution_accuracy > 0) || !(cfg->scale > 0))
+        return rs_set_error("rs_maps_replay: resolution_accuracy / scale must be positive");
+    if (!st->visit_lut) return rs_set_error("rs_maps_replay: RsMapsState.visit_lut is NULL");
+    if (!obs_rows || !end_rows) return rs_set_error("rs_maps_replay: obs_rows / end_rows is NULL");
+    if (m == 0) return 0;
+    if (!ranges || !out_row0 || !out_actor || !out_critic || !out_status)
+        return rs_set_error("rs_maps_replay: ranges / out_row0 / out_actor / out_critic / out_status is NULL");
+    const int grid = (m + kWarpsPerBlock - 1) / kWarpsPerBlock;
+    const size_t smem = (size_t)kWarpsPerBlock * cfg->log_cap * (2 * sizeof(float) + sizeof(uint16_t)) + 16;
+    if (smem > 48 * 1024)
+        cudaFuncSetAttribute(maps_replay_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    maps_replay_kernel<<<grid, kBlock, smem, static_cast<cudaStream_t>(stream)>>>(
+        *cfg, st->visit_lut, obs_rows, pred_rows, end_rows, T, n_env, ranges, m, out_row0, out_actor, out_critic, out_status);
     return (int)cudaGetLastError();
 }
 

@@ -8,7 +8,9 @@ z-score), visit counts (log-scale normalised), obstacle detections, and the comb
 
 `BatchedMapsBuffer` holds the stacks of all N environments x A agents persistently in HBM and updates them sparsely in
 place with one kernel launch per call (rs_maps_update / rs_maps_reset, include/radsearch_b200.h); the tensors it returns
-are those persistent stacks.  `MapsBuffer` is the single-buffer form with the reference's method names.
+are those persistent stacks.  `replay` rebuilds the stacks the policy saw at any (env, step) of a rollout buffer for the
+PPO update (rs_maps_replay): storing them is out of reach at batch scale (4*(6A+4)*X*Y bytes per env and step, 81.6 KB at
+A = 4), their inputs are already in the buffer.  `MapsBuffer` is the single-buffer form with the reference's method names.
 There is no CPU path.
 """
 from __future__ import annotations
@@ -120,6 +122,51 @@ class BatchedMapsBuffer:
         with torch.cuda.device(self.device):
             L.check(self._lib.rs_maps_reset(C.byref(self._cfg), C.byref(self._st), _ptr(m), int(mask_bits),
                                             self.num_envs, self._stream()), "rs_maps_reset")
+
+
+    def replay(self, buf, ranges: torch.Tensor, out: Optional[Tuple[torch.Tensor, torch.Tensor]] = None):
+        """The stacks the policy read during the collection of `buf` (a BatchedPPOBuffer made with agents=A, filled by
+        TeamRolloutCollector), for the requested ranges: int32 [M, 3] rows (env n, first step t0, last step t1), e.g.
+        episode_ranges(...) of pack_episodes().  Range i fills rows sum(len[:i]) .. + len[i] - 1, len = t1 - t0 + 1 (0 for
+        an inverted range).  Returns (actor [R, A, 6, X, Y], critic [R, 4, X, Y]) -- channels_last views like the live
+        stacks -- and status int32 [M]: the RS_MS_* bits of the replayed calls, | MR_BAD_RANGE (8) for a range outside the
+        buffer (zero stacks) or inverted.  `out`: (actor store [R, A, X, Y, 6], critic store [R, X, Y, 4]) float32 to fill
+        (no host synchronisation then; otherwise R is read back once).  The live state is neither read nor written."""
+        if buf.A != self.number_of_agents or buf.num_envs != self.num_envs or buf.D != L.OBS_DIM:
+            raise ValueError("replay needs a BatchedPPOBuffer(11, T, num_envs, agents=number_of_agents) of this batch")
+        A, (X, Y) = self.number_of_agents, self.map_dimensions
+        rg = ranges.to(device=self.device, dtype=torch.int32).reshape(-1, 3).contiguous()
+        m = rg.shape[0]
+        lens = (rg[:, 2].long() - rg[:, 1].long() + 1).clamp(min=0)
+        row0 = (torch.cumsum(lens, 0) - lens).contiguous()
+        if out is None:
+            R = int(lens.sum().item()) if m else 0
+            a_store = torch.empty(R, A, X, Y, 6, dtype=torch.float32, device=self.device)
+            c_store = torch.empty(R, X, Y, 4, dtype=torch.float32, device=self.device)
+        else:
+            a_store, c_store = out
+            R = a_store.shape[0]
+            if a_store.shape != (R, A, X, Y, 6) or c_store.shape != (R, X, Y, 4) or not a_store.is_contiguous() or \
+                    not c_store.is_contiguous() or a_store.dtype != torch.float32 or c_store.dtype != torch.float32:
+                raise ValueError("out must be contiguous float32 stores [R, A, X, Y, 6] and [R, X, Y, 4]")
+        status = torch.zeros(m, dtype=torch.int32, device=self.device)
+        with torch.cuda.device(self.device):
+            L.check(self._lib.rs_maps_replay(C.byref(self._cfg), C.byref(self._st), _ptr(buf._obs_store), _ptr(buf.pred_buf),
+                                             _ptr(buf.end_buf), buf.T, self.num_envs, _ptr(rg), m, _ptr(row0),
+                                             _ptr(a_store), _ptr(c_store), _ptr(status), self._stream()), "rs_maps_replay")
+        return a_store.permute(0, 1, 4, 2, 3), c_store.permute(0, 3, 1, 2), status
+
+
+def episode_ranges(ep_start: torch.Tensor, ep_len: torch.Tensor, steps_per_epoch: int, agents: int = 1) -> torch.Tensor:
+    """Replay ranges int32 [E', 3] = (env, t0, t1) of the episodes of a BatchedPPOBuffer.pack_episodes() table.  With
+    agents=A the table lists every episode once per agent column (n*A + a) and the A columns of an env end together: the
+    episodes of agent 0's columns are kept, once per env, in (env, time) order."""
+    T = int(steps_per_epoch)
+    col = ep_start.long() // T
+    t0 = ep_start.long() - col * T
+    keep = (col % agents) == 0
+    col, t0, n_steps = col[keep], t0[keep], ep_len.long()[keep]
+    return torch.stack((col // agents, t0, t0 + n_steps - 1), dim=1).to(torch.int32).contiguous()
 
 
 class MapsBuffer:

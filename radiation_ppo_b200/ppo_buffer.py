@@ -206,13 +206,22 @@ class BatchedPPOBuffer:
     store_batch() appends one step for every column; `end`/`boot` carry the caller rules of train.py:446-491
     (end[t, n] != 0 where the reference would call GAE_advantage_and_rewardsToGO after step t, boot[t, n] the bootstrap
     value passed there).  finish_paths() is one rs_gae launch; get() normalises the advantages with the global
-    (all-rank) statistics."""
+    (all-rank) statistics.
+
+    ``agents=A`` (RAD-TEAM, TeamRolloutCollector): `num_columns` counts environments and the buffer has N*A env-major
+    columns (column n*A + a, the memory order of the env's [N, A] outputs), plus `pred_buf` [T, N*A, 2], the PFGRU's
+    source predictions the map observation was updated with (what BatchedMapsBuffer.replay needs besides the
+    observations and path ends).  GAE runs per column; agent_view() gives the [T, N] per-agent slices."""
 
     def __init__(self, observation_dimension: int, steps_per_epoch: int, num_columns: int, gamma: float = 0.99,
-                 lam: float = 0.90, device=None) -> None:
+                 lam: float = 0.90, device=None, agents: Optional[int] = None) -> None:
         self.device = _need_cuda(device)
         L.load()
-        T, N, D = steps_per_epoch, num_columns, observation_dimension
+        if agents is not None and not 1 <= int(agents) <= L.MAX_A:
+            raise ValueError("agents must be in 1..8")
+        self.A = None if agents is None else int(agents)
+        self.num_envs = num_columns
+        T, N, D = steps_per_epoch, num_columns * (self.A or 1), observation_dimension
         self.T, self.N, self.D = T, N, D
         self.gamma, self.lam = gamma, lam
         z = lambda *s, dt=torch.float32: torch.zeros(*s, dtype=dt, device=self.device)   # noqa: E731
@@ -226,6 +235,7 @@ class BatchedPPOBuffer:
         self.boot_buf = z(T, N)
         self.end_buf = z(T, N, dt=torch.uint8)
         self.source_tar = z(T, N, 2)
+        self.pred_buf = None if self.A is None else torch.full((T, N, 2), float("nan"), dtype=torch.float32, device=self.device)
         self.stats = z(2, dt=torch.float64)
         self.ptr = 0
 
@@ -246,13 +256,33 @@ class BatchedPPOBuffer:
         non-zero exactly where train.py:446-491 finishes a trajectory) -> end_buf[t]."""
         t = self.ptr if t is None else t
         assert 0 <= t < self.T
+        if self.A is not None:
+            # the env's reward [N, A] / ended [N] are not the rows' layout (team reward rule, A path-end bytes per env):
+            # rs_rollout_post_team writes those rows
+            return {"obs": self._obs_store[t + 1]}
         return {"obs": self._obs_store[t + 1], "reward": self.rew_buf[t], "ended": self.end_buf[t]}
 
     def policy_rows(self, t: Optional[int] = None) -> Dict[str, torch.Tensor]:
         """Rows of step t the policy side fills: obs (read), act / val / logp / boot / src (write)."""
         t = self.ptr if t is None else t
-        return {"obs": self._obs_store[t], "act": self.act_buf[t], "val": self.val_buf[t], "logp": self.logp_buf[t],
+        rows = {"obs": self._obs_store[t], "act": self.act_buf[t], "val": self.val_buf[t], "logp": self.logp_buf[t],
                 "boot": self.boot_buf[t], "src": self.source_tar[t]}
+        if self.A is not None:
+            rows.update(pred=self.pred_buf[t], rew=self.rew_buf[t], end=self.end_buf[t])
+        return rows
+
+    def agent_view(self, a: int) -> Dict[str, torch.Tensor]:
+        """Agent a's columns of a buffer made with ``agents=A``: [T, N] (obs [T, N, D], src / pred [T, N, 2]) strided views
+        of obs / act / rew / val / logp / adv / ret / boot / end / src / pred, for a per-agent update."""
+        if self.A is None:
+            raise ValueError("agent_view needs a buffer made with agents=A")
+        if not 0 <= a < self.A:
+            raise ValueError("agent index out of range")
+        T, N, A = self.T, self.num_envs, self.A
+        v = lambda x: x.reshape(T, N, A, *x.shape[2:])[:, :, a]                  # noqa: E731
+        return dict(obs=v(self.obs_buf), act=v(self.act_buf), rew=v(self.rew_buf), val=v(self.val_buf),
+                    logp=v(self.logp_buf), adv=v(self.adv_buf), ret=v(self.ret_buf), boot=v(self.boot_buf),
+                    end=v(self.end_buf), src=v(self.source_tar), pred=v(self.pred_buf))
 
     def advance(self) -> None:
         assert self.ptr < self.T

@@ -53,10 +53,13 @@ class EpisodeStats:
         self.steps_in_episode.masked_fill_(reset, 0)
 
     def fused_args(self):
-        """Device pointers of the single-agent accumulators for rs_rollout_post (which does what `update` does, in the
-        same launch as the bootstrap rule): ep_return [N] f64, ep_steps [N] i32, acc [6] f64, min [1], max [1]."""
-        if self.A != 1 or self.team_mode == "competitive":
-            raise ValueError("the fused bookkeeping covers one agent per environment")
+        """The accumulators for rs_rollout_post / rs_rollout_post_team (which do what `update` does, in the same launch as
+        the bootstrap rule): ep_return [N, A] f64, ep_steps [N] i32, acc [6, A] f64, min [A], max [A].  The fused kernels
+        implement the 'individual' rule (each agent's own reward) and the team reward of the other modes except
+        'competitive'."""
+        if self.team_mode == "competitive":
+            raise ValueError("the fused bookkeeping covers one agent per environment or the individual / cooperative "
+                             "reward rules")
         return (self.episode_return, self.steps_in_episode, self._acc, self._min, self._max)
 
     def epoch_summary(self, group=None, clear: bool = True) -> Dict[str, torch.Tensor]:
