@@ -240,6 +240,22 @@ int rs_rollout_post_team(const float *reward, const float *team_reward, const ui
                          uint8_t *end_row, int32_t n_env, int32_t n_agents, int32_t individual, int32_t last_step,
                          void *stream);
 
+/* ---- caller-side bookkeeping of the batched Monte-Carlo evaluation (algos/multiagent/evaluate.py:333-475), one elementwise
+ * launch per step ------------------------------------------------------------------------------------------------------
+ * rs_eval_step, after the env step (auto-reset off), for every env n with active[n] != 0 on entry (the others are not
+ * touched): length[n] += 1; ep_return[n][a] += individual ? reward[n][a] : team_reward[n] (float32 rewards summed in
+ * float64, E:402-409); oob[n][a] += (info[n][a] & RS_I_OOB) != 0; when any done[n][a] != 0 (E:415-419): success[n] = 1,
+ * active[n] = 0, finders[n] = bit mask of those agents (nullable) and *n_active -= 1 (one atomic per warp).
+ * Localisation error (an addition, not a field of the reference's MonteCarloResults; nullable as a group): where pred
+ * [N][A][2] (the policy's source prediction of the step in scaled coordinates) is not NaN, e = hypot(pred / scale - src)
+ * in fp64 cm with src [N][2] int32 and scale = the env's coordinate scale; loc_err_sum[n][a] += e, loc_err_n[n][a] += 1,
+ * loc_err_last[n][a] = (float)e.  active / success / finders u8 [N], length i32 [N], ep_return f64 [N][A], oob i32 [N][A],
+ * n_active i32 [1], loc_err_sum f64 / loc_err_n i32 / loc_err_last f32 [N][A]. */
+int rs_eval_step(const float *reward, const float *team_reward, const uint8_t *done, const uint8_t *info, uint8_t *active,
+                 uint8_t *success, int32_t *length, double *ep_return, int32_t *oob, uint8_t *finders, int32_t *n_active,
+                 const float *pred, const int32_t *src, double scale, double *loc_err_sum, int32_t *loc_err_n,
+                 float *loc_err_last, int32_t n_env, int32_t n_agents, int32_t individual, void *stream);
+
 /* ---- RAD-TEAM map observation (SURVEY.md 8f-1) ---------------------------------------------------------------------
  * MapsBuffer.observation_to_map (algos/multiagent/NeuralNetworkCores/RADTEAM_core.py:532-616 with its helpers :101-182
  * IntensityEstimator, :188-277 StatisticStandardization, :322-365 log-scale normalisation, :692-932 map updates) for

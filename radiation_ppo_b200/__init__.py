@@ -11,10 +11,12 @@ from .ppo_buffer import (BatchedPPOBuffer, PPOBuffer, advantage_statistics, comb
                          normalize_advantages_)
 from .dist import shard_range
 from .maps_buffer import BatchedMapsBuffer, MapsBuffer, episode_ranges
-from .evaluate import MonteCarloEvaluator, MonteCarloResults, uniform_policy
+from .evaluate import (MonteCarloEvaluator, MonteCarloResults, TeamEvalPolicy, TeamMonteCarloResults,
+                       uniform_policy)
 from .rollout_stats import EpisodeStats
 from .rollout import RolloutCollector, TeamRolloutCollector, TeamRolloutPolicy
 
 __all__ = ["RadSearch", "StepResult", "HostStepBuffers", "PPOBuffer", "BatchedPPOBuffer", "gae_advantages", "advantage_statistics",
-           "normalize_advantages_", "combined_shape", "shard_range", "BatchedMapsBuffer", "MapsBuffer", "MonteCarloEvaluator", "MonteCarloResults", "uniform_policy", "EpisodeStats", "RolloutCollector",
+           "normalize_advantages_", "combined_shape", "shard_range", "BatchedMapsBuffer", "MapsBuffer", "MonteCarloEvaluator", "MonteCarloResults", "TeamMonteCarloResults",
+           "TeamEvalPolicy", "uniform_policy", "EpisodeStats", "RolloutCollector",
            "TeamRolloutCollector", "TeamRolloutPolicy", "episode_ranges", "RadSearchLibraryError", "_lib"]

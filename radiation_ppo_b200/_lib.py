@@ -21,7 +21,7 @@ EXPORTS = [
     "rs_step", "rs_reset", "rs_prepare", "rs_bump_ctr", "rs_load_scenarios", "rs_query_shortest_path", "rs_gae", "rs_adv_stats", "rs_adv_normalize", "rs_last_error",
     "rs_version", "rs_sizeof_config", "rs_sizeof_state", "rs_maps_update", "rs_maps_reset", "rs_sizeof_maps_config",
     "rs_sizeof_maps_state", "rs_pack_rollout", "rs_episode_table", "rs_rollout_pre", "rs_rollout_post",
-    "rs_rollout_pre_team", "rs_rollout_post_team", "rs_maps_replay",
+    "rs_rollout_pre_team", "rs_rollout_post_team", "rs_maps_replay", "rs_eval_step",
 ]
 MS_CELL_RANGE, MS_LOG_FULL, MS_PRED_RANGE = 1, 2, 4
 MR_BAD_RANGE = 8
@@ -123,6 +123,8 @@ def declare(lib, prefix="rs_"):
                                              vp]
         lib.rs_maps_replay.restype = i32
         lib.rs_maps_replay.argtypes = [mcp, msp, vp, vp, vp, i32, i32, vp, i32, vp, vp, vp, vp, vp]
+        lib.rs_eval_step.restype = i32
+        lib.rs_eval_step.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, f64, vp, vp, vp, i32, i32, i32, vp]
         lib.rs_sizeof_maps_config.restype = i32
         lib.rs_sizeof_maps_state.restype = i32
         lib.rs_last_error.restype = C.c_char_p
