@@ -270,7 +270,9 @@ typedef struct RsMapsConfig {
     int32_t n_agents;            /* A                                                                    :437      */
     int32_t dim_x, dim_y;        /* map_dimensions (27 x 27 with enforced boundaries, 147 x 147 without) :60-66    */
     int32_t base;                /* (steps_per_episode + 1) * A: base of the visit-count normalisation   :500      */
-    int32_t log_cap;             /* readings an episode can record per environment (>= base + A)                   */
+    int32_t log_cap;             /* readings an episode can record per environment (>= base + A, <= 5810: the     */
+                                 /* kernels keep 4 tables in one block's shared memory, 40 * log_cap + 16 bytes,  */
+                                 /* and sm_100 allows 227 KB)                                                     */
     int32_t use_prediction;      /* PFGRU: maintain the source prediction map                            :39       */
     double resolution_accuracy;  /* resolution_multiplier / scale (22.0)                                 :69-70    */
     double scale;                /* the environment's coordinate scale 1 / search_area_max  rad_search_env.py:435  */

@@ -30,6 +30,18 @@ namespace {
 
 constexpr int kWarpsPerBlock = 4;
 constexpr int kBlock = 32 * kWarpsPerBlock;
+// Dynamic shared memory of maps_update_kernel / maps_replay_kernel: per warp the sample table (value, cell) and the
+// compaction scratch, 10 bytes per reading.  A block of sm_100 gets at most 227 KB, so log_cap <= 5810.
+constexpr size_t kMaxSmemPerBlock = 227 * 1024;
+constexpr int kMaxLogCap =
+    (int)((kMaxSmemPerBlock - 16) / (kWarpsPerBlock * (2 * sizeof(float) + sizeof(uint16_t))));
+#define RS_LOG_CAP_MSG "log_cap out of range [n_agents, 5810]: 40 * log_cap + 16 bytes of shared memory per block " \
+                       "exceed the 227 KB (232448 bytes) of sm_100"
+static_assert(kMaxLogCap == 5810, "RS_LOG_CAP_MSG names the limit");
+
+size_t maps_smem_bytes(int log_cap) {
+    return (size_t)kWarpsPerBlock * log_cap * (2 * sizeof(float) + sizeof(uint16_t)) + 16;
+}
 
 __device__ __forceinline__ int cell_of(const RsMapsConfig &c, double vx, double vy) {
     // int(v * resolution_accuracy) M:704-713, then numpy indexing: negative indices wrap once
@@ -414,7 +426,7 @@ int check_maps(const RsMapsConfig *c, const RsMapsState *s, int32_t n_env) {
     if (n_env <= 0) return rs_set_error("n_env must be positive");
     if (c->n_agents < 1 || c->n_agents > RS_MAX_A) return rs_set_error("n_agents out of range [1, 8]");
     if (c->dim_x < 1 || c->dim_y < 1 || (int64_t)c->dim_x * c->dim_y > 65535) return rs_set_error("map dimensions out of range");
-    if (c->log_cap < c->n_agents || c->log_cap > 8192) return rs_set_error("log_cap out of range");
+    if (c->log_cap < c->n_agents || c->log_cap > kMaxLogCap) return rs_set_error(RS_LOG_CAP_MSG);
     if (c->base < 2) return rs_set_error("base must be >= 2");
     if (!(c->resolution_accuracy > 0) || !(c->scale > 0)) return rs_set_error("resolution_accuracy / scale must be positive");
     if (!s->actor || !s->critic || !s->log_cell || !s->log_val || !s->log_len || !s->last_cell ||
@@ -432,9 +444,11 @@ int rs_maps_update(const RsMapsConfig *cfg, const RsMapsState *st, const float *
     if (int rc = check_maps(cfg, st, n_env)) return rc;
     if (!obs) return rs_set_error("obs is NULL");
     const int grid = (n_env + kWarpsPerBlock - 1) / kWarpsPerBlock;
-    const size_t smem = (size_t)kWarpsPerBlock * cfg->log_cap * (2 * sizeof(float) + sizeof(uint16_t)) + 16;
-    if (smem > 48 * 1024)
-        cudaFuncSetAttribute(maps_update_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    const size_t smem = maps_smem_bytes(cfg->log_cap);
+    if (smem > 48 * 1024) {
+        const cudaError_t e = cudaFuncSetAttribute(maps_update_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return (int)e;
+    }
     maps_update_kernel<<<grid, kBlock, smem, static_cast<cudaStream_t>(stream)>>>(*cfg, *st, obs, loc_pred, mask,
                                                                                   mask_bits ? mask_bits : 0xff, n_env);
     return (int)cudaGetLastError();
@@ -458,7 +472,7 @@ int rs_maps_replay(const RsMapsConfig *cfg, const RsMapsState *st, const float *
     if (cfg->n_agents < 1 || cfg->n_agents > RS_MAX_A) return rs_set_error("rs_maps_replay: n_agents out of range [1, 8]");
     if (cfg->dim_x < 1 || cfg->dim_y < 1 || (int64_t)cfg->dim_x * cfg->dim_y > 65535)
         return rs_set_error("rs_maps_replay: map dimensions out of range");
-    if (cfg->log_cap < cfg->n_agents || cfg->log_cap > 8192) return rs_set_error("rs_maps_replay: log_cap out of range");
+    if (cfg->log_cap < cfg->n_agents || cfg->log_cap > kMaxLogCap) return rs_set_error("rs_maps_replay: " RS_LOG_CAP_MSG);
     if (!(cfg->resolution_accuracy > 0) || !(cfg->scale > 0))
         return rs_set_error("rs_maps_replay: resolution_accuracy / scale must be positive");
     if (!st->visit_lut) return rs_set_error("rs_maps_replay: RsMapsState.visit_lut is NULL");
@@ -467,9 +481,11 @@ int rs_maps_replay(const RsMapsConfig *cfg, const RsMapsState *st, const float *
     if (!ranges || !out_row0 || !out_actor || !out_critic || !out_status)
         return rs_set_error("rs_maps_replay: ranges / out_row0 / out_actor / out_critic / out_status is NULL");
     const int grid = (m + kWarpsPerBlock - 1) / kWarpsPerBlock;
-    const size_t smem = (size_t)kWarpsPerBlock * cfg->log_cap * (2 * sizeof(float) + sizeof(uint16_t)) + 16;
-    if (smem > 48 * 1024)
-        cudaFuncSetAttribute(maps_replay_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    const size_t smem = maps_smem_bytes(cfg->log_cap);
+    if (smem > 48 * 1024) {
+        const cudaError_t e = cudaFuncSetAttribute(maps_replay_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return (int)e;
+    }
     maps_replay_kernel<<<grid, kBlock, smem, static_cast<cudaStream_t>(stream)>>>(
         *cfg, st->visit_lut, obs_rows, pred_rows, end_rows, T, n_env, ranges, m, out_row0, out_actor, out_critic, out_status);
     return (int)cudaGetLastError();

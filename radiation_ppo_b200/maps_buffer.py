@@ -24,6 +24,9 @@ import torch
 
 from . import _lib as L
 
+# readings an episode's sample table can hold: the map kernels keep 4 warps' tables in one block's shared memory,
+# 40 * log_cap + 16 bytes, and sm_100 allows 227 KB (rs_maps.cu)
+MAX_LOG_CAP = 5810
 ACTOR_MAPS = ("prediction", "location", "others_locations", "readings", "visit_counts", "obstacles")   # M:1811-1820
 CRITIC_MAPS = ("combined_location", "readings", "visit_counts", "obstacles")                            # M:1825-1832
 
@@ -64,6 +67,11 @@ class BatchedMapsBuffer:
         self.base = (self.steps_per_episode + 1) * self.number_of_agents                               # M:500
         N, A, (X, Y) = self.num_envs, self.number_of_agents, self.map_dimensions
         cap = self.base + 2 * A              # one call per step, the reset observation and the bootstrap call
+        if cap > MAX_LOG_CAP:
+            raise ValueError(f"steps_per_episode={self.steps_per_episode} with number_of_agents={A}: the sample table "
+                             f"holds (steps_per_episode + 3) * number_of_agents = {cap} readings, at most {MAX_LOG_CAP} "
+                             f"fit the 227 KB of shared memory a block of the map kernels gets on sm_100 "
+                             f"(steps_per_episode <= {MAX_LOG_CAP // A - 3} at {A} agents)")
         cfg = L.RsMapsConfig()
         cfg.n_agents, cfg.dim_x, cfg.dim_y, cfg.base, cfg.log_cap = A, X, Y, self.base, cap
         cfg.use_prediction = int(bool(use_prediction))

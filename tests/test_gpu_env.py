@@ -29,7 +29,8 @@ def make_pair(n, A=1, oc=5, enforce=True, seed=11, env_id0=3, max_ep_len=120, **
 @pytest.mark.parametrize("n,A,oc,enforce,T,idle", [(1024, 1, 5, True, 130, 0.0), (1024, 1, -1, False, 100, 0.0),
                                                    (512, 4, 5, True, 90, 0.15), (256, 1, 0, True, 40, 0.0),
                                                    (300, 2, 7, True, 70, 0.1), (37, 1, 3, False, 50, 0.0),
-                                                   (480, 3, 4, True, 80, 0.1), (96, 5, 2, True, 40, 0.2), (50, 8, 3, True, 30, 0.1)])
+                                                   (480, 3, 4, True, 80, 0.1), (96, 5, 2, True, 40, 0.2), (50, 8, 3, True, 30, 0.1),
+                                                   (200, 6, 4, True, 40, 0.1), (77, 7, 6, False, 40, 0.15)])
 def test_rollout_matches_oracle(n, A, oc, enforce, T, idle):
     env, ob = make_pair(n, A, oc, enforce, seed=100 + n)
     v = pu.GpuView(env)

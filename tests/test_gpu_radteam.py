@@ -117,7 +117,9 @@ def check_replay(mb, buf, pol, sample, T, rng):
 
 
 @pytest.mark.parametrize("A,mode,team_mode", [(1, "rows", "cooperative"), (1, "graph", "individual")] +
-                         [(A, m, tm) for A in (2, 4) for m in ("rows", "graph") for tm in ("individual", "cooperative")])
+                         [(A, m, tm) for A in (2, 4) for m in ("rows", "graph") for tm in ("individual", "cooperative")] +
+                         [(3, "rows", "individual"), (6, "graph", "cooperative"), (8, "rows", "cooperative"),
+                          (8, "graph", "individual")])
 def test_team_collector_epoch_matches_oracle_and_replay(A, mode, team_mode):
     """Two epochs of TeamRolloutCollector against the oracle env stepped the reference's way: observation rows, rewards per
     team mode, path ends in all A columns, actions, source coordinates, predictions, the bootstrap rule, GAE, the

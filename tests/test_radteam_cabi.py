@@ -91,6 +91,39 @@ def test_maps_replay_argument_errors(lib):
         setattr(mc, field, old)
 
 
+def test_maps_log_cap_bounded_by_shared_memory(lib):
+    """The update and replay kernels keep 4 sample tables of 10 bytes per reading (+ 16 bytes) in one block's shared
+    memory, and sm_100 gives a block 227 KB (232448 bytes): log_cap 5810 is the largest that fits.  A larger one is an
+    argument error of rs_maps_update, rs_maps_reset and rs_maps_replay, found before any CUDA call; 5810 passes the check
+    (each call below then fails a later check, so nothing is launched)."""
+    d = DUMMY
+    mc, ms = maps_cfg()
+    mc.n_agents = 8
+    for k in ("actor", "critic", "log_cell", "log_val", "log_len", "last_cell", "last_pred", "std", "std_count", "status"):
+        setattr(ms, k, d.value)
+
+    def update(obs=d):
+        return lib.rs_maps_update(C.byref(mc), C.byref(ms), obs, None, None, 0, 16, None)
+
+    def reset():
+        return lib.rs_maps_reset(C.byref(mc), C.byref(ms), None, 0, 16, None)
+
+    def replay():
+        return lib.rs_maps_replay(C.byref(mc), C.byref(ms), d, d, d, 48, 16, d, 4, d, d, d, d, None)
+
+    for cap in (5811, 8192):
+        mc.log_cap = cap
+        for f in (update, reset, replay):
+            assert f() < 0, (cap, f.__name__)
+            assert "log_cap" in err(lib) and "5810" in err(lib) and "232448" in err(lib), (cap, f.__name__)
+    mc.log_cap = 5810
+    assert update(obs=None) < 0 and err(lib) == "obs is NULL"
+    ms.status = None
+    assert reset() < 0 and "NULL members" in err(lib)
+    ms.visit_lut = None
+    assert replay() < 0 and "visit_lut" in err(lib)
+
+
 def test_episode_ranges_from_an_episode_table():
     """pack_episodes' table of an agents=2 buffer (columns n*2 + a, T = 10): every episode appears once per agent
     column; the ranges keep agent 0's, as (env, t0, t1)."""
