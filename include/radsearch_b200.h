@@ -172,13 +172,16 @@ int rs_query_shortest_path(const RsConfig *cfg, const RsState *st, const int32_t
 /* GAE-lambda advantages and rewards-to-go over a [T][N] rollout.  path_end[t][n] != 0 where the caller finished a
  * trajectory after step t; boot[t][n] = bootstrap value passed there (read only where path_end or t == T-1).
  * stats (nullable): double[2] device accumulators += {sum(adv), sum(adv^2)} (zero them first).
- * variant: 0 auto; 1 thread-per-column recurrence in the reference's operation order (bit-exact vs scipy's lfilter), fed by
- * bulk-async tile copies when N % 128 == 0 and the arrays are 16-byte aligned, else by register-pipelined loads; 2 warp-
- * shuffle scan along T (small N; within 1e-5).  3 / 4 force the 8- / 16-deep register-pipelined form, 7 the 3-stage tile
- * ring, 10 the same ring over 64-column tiles, 8 / 11 the producer-warp form with 3 x 8 and 6 x 8 rows in flight, 12 / 13
- * that form over 64- / 224-column tiles, 14 / 15 the producer-warp form fed by tensor-map (2-D TMA) copies over 128- /
- * 224-column tiles -- all bit-identical to variant 1.  Auto: N >= 75776 -> 7, N >= 32768 -> 13, N >= 16384 -> 14 (whole
- * tiles), N < 16384 -> 2. */
+ * variant (defined: 0-4, 7, 8, 10-15; any other number is an argument error): 0 auto; 1 thread-per-column recurrence in the
+ * reference's operation order (bit-exact vs scipy's lfilter), fed by bulk-async tile copies when N % 128 == 0 and the
+ * arrays are 16-byte aligned, else by register-pipelined loads; 2 warp-shuffle scan along T (small N; each output within
+ * one float32 ulp of the float64 recurrence; T * 104 bytes of shared memory, at most 227 KB).  3 / 4 force the 8- / 16-deep
+ * register-pipelined form, 7 the 3-stage tile ring, 10 the same ring over 64-column tiles, 8 / 11 the producer-warp form
+ * with 3 x 8 and 6 x 8 rows in flight, 12 / 13 that form over 64- / 224-column tiles, 14 / 15 the producer-warp form fed
+ * by tensor-map (2-D TMA) copies over 128- / 224-column tiles -- all bit-identical to variant 1.  Variants 7-15 need whole
+ * tiles (N % 128 == 0, 16-byte aligned rew / val / path_end).  Auto, with whole tiles: N >= 75776 -> 7, N >= 32768 -> 13,
+ * N >= 16384 -> 14; N < 16384 with T * 104 <= 200 KB -> 2; otherwise the register-pipelined form, 8-deep when N > 75776.
+ * Variant 1 is auto without the scan. */
 int rs_gae(const float *rew, const float *val, const uint8_t *path_end, const float *boot, float *adv, float *ret,
            int32_t T, int32_t N, double gamma, double lam, double *stats, int32_t variant, void *stream);
 

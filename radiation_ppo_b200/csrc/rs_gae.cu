@@ -92,7 +92,7 @@ __global__ void __launch_bounds__(kColsBlock, MINB) gae_cols_kernel(const float 
 }
 
 // ------------------------------------------------------------------------------------------------------------------
-// variant 6: the same per-column recurrence (same operation order: bit-identical to variant 1) fed by the copy engine.
+// variants 7 / 10: the same per-column recurrence (same operation order: bit-identical to variant 1) fed by the copy engine.
 // A CTA owns 128 columns; the [U rows][128 columns] tiles of rew / val / path_end travel HBM -> shared memory as
 // bulk-async copies (cp.async.bulk + mbarrier, one 512-byte / 128-byte run per row) through a ring of S stages issued S
 // chunks ahead, so the threads spend their instructions on the fp64 chain instead of on address arithmetic and on
@@ -254,7 +254,7 @@ __global__ void __launch_bounds__(C, MINB) gae_tile_kernel(const float *__restri
     }
 }
 
-// variant 8: variant 6/7 with a producer warp.  Warp 4 only refills stages (it waits on the stage's `empty` barrier, which
+// variants 8 / 11 / 12 / 13: variant 7 with a producer warp.  Warp 4 only refills stages (it waits on the stage's `empty` barrier, which
 // the 128 consumer threads arrive on when they are done reading it), so no CTA-wide barrier sits in the consumers' loop
 // and the four consumer warps drift apart by up to S chunks.
 template <int C, int U, int S, int MINB>
@@ -651,14 +651,17 @@ int rs_gae(const float *rew, const float *val, const uint8_t *path_end, const fl
            int32_t T, int32_t N, double gamma, double lam, double *stats, int32_t variant, void *stream) {
     if (!rew || !val || !path_end || !boot || !adv || !ret) return rs_set_error("rs_gae: NULL buffer");
     if (T <= 0 || N <= 0) return rs_set_error("rs_gae: T and N must be positive");
+    if (variant < 0 || variant > 15 || variant == 5 || variant == 6 || variant == 9) return rs_set_error("rs_gae: unknown variant");
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const double gl = gamma * lam;
     const size_t scan_smem = (size_t)T * kTileCols * (3 * sizeof(float) + 1);
     if (variant == 0) variant = (N < 16384 && scan_smem <= 200 * 1024) ? 2 : 1;
     if (variant == 2) {
         if (scan_smem > 227 * 1024) return rs_set_error("rs_gae: T too large for the scan variant");
-        if (scan_smem > 48 * 1024)
-            cudaFuncSetAttribute(gae_scan_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)scan_smem);
+        if (scan_smem > 48 * 1024) {
+            const cudaError_t e = cudaFuncSetAttribute(gae_scan_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)scan_smem);
+            if (e != cudaSuccess) return (int)e;
+        }
         const int grid = (N + kTileCols - 1) / kTileCols;
         gae_scan_kernel<<<grid, kScanBlock, scan_smem, s>>>(rew, val, path_end, boot, adv, ret, T, N, gamma, gl, stats);
     } else {
@@ -690,7 +693,9 @@ int rs_gae(const float *rew, const float *val, const uint8_t *path_end, const fl
 #define RS_GAE_WS(CW, MINB)                                                                                                \
     do {                                                                                                                   \
         constexpr int sm = 9 * 6 * 8 * CW + 2 * 6 * 8;                                                                     \
-        cudaFuncSetAttribute(gae_tile_ws_kernel<CW, 8, 6, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm);         \
+        const cudaError_t e = cudaFuncSetAttribute(gae_tile_ws_kernel<CW, 8, 6, MINB>,                                     \
+                                                   cudaFuncAttributeMaxDynamicSharedMemorySize, sm);                       \
+        if (e != cudaSuccess) return (int)e;                                                                               \
         gae_tile_ws_kernel<CW, 8, 6, MINB><<<(N + CW - 1) / CW, CW + 32, sm, s>>>(rew, val, path_end, boot, adv, ret, T, N, \
                                                                               gamma, gl, stats);                          \
     } while (0)
@@ -706,7 +711,9 @@ int rs_gae(const float *rew, const float *val, const uint8_t *path_end, const fl
             !make_tmap(&tp, path_end, true, T, N, 8, CW))                                                                  \
             return rs_set_error("rs_gae: cuTensorMapEncodeTiled failed");                                                  \
         constexpr int sm = 9 * 6 * 8 * CW + 2 * 6 * 8;                                                                     \
-        cudaFuncSetAttribute(gae_tmap_kernel<CW, 8, 6, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm);            \
+        const cudaError_t e = cudaFuncSetAttribute(gae_tmap_kernel<CW, 8, 6, MINB>,                                        \
+                                                   cudaFuncAttributeMaxDynamicSharedMemorySize, sm);                       \
+        if (e != cudaSuccess) return (int)e;                                                                               \
         gae_tmap_kernel<CW, 8, 6, MINB><<<(N + CW - 1) / CW, CW + 32, sm, s>>>(tr, tv, tp, boot, adv, ret, T, N, gamma, gl, \
                                                                            stats);                                        \
     } while (0)

@@ -78,7 +78,10 @@ int rs_pack_rollout(const float *obs, const float *adv, const float *ret, const 
     if (T <= 0 || N <= 0 || D <= 0 || D > 64) return rs_set_error("rs_pack_rollout: bad T / N / D");
     const dim3 grid((N + kTN - 1) / kTN, (T + kTT - 1) / kTT);
     const size_t smem = (size_t)kTN * kTT * (D + 6) * sizeof(float);
-    if (smem > 48 * 1024) cudaFuncSetAttribute(pack_rollout_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (smem > 48 * 1024) {
+        const cudaError_t e = cudaFuncSetAttribute(pack_rollout_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return (int)e;
+    }
     pack_rollout_kernel<<<grid, kPackBlock, smem, static_cast<cudaStream_t>(stream)>>>(obs, adv, ret, logp, act, src, packed,
                                                                                       T, N, D);
     return (int)cudaGetLastError();
