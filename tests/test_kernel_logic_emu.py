@@ -13,14 +13,39 @@ from tests.emu.harness import EmuEnv, make_config
 compare_state, compare_obs = pu.compare_state, pu.compare_obs
 
 
-@pytest.mark.parametrize("n,A,oc,enforce,T,idle", [(192, 1, 5, True, 130, 0.0), (128, 1, -1, False, 90, 0.0),
-                                                   (96, 3, 4, True, 80, 0.2), (64, 1, 0, True, 40, 0.0),
-                                                   (48, 2, 7, True, 60, 0.1)])
-def test_emulated_kernels_match_oracle_rollout(n, A, oc, enforce, T, idle):
+_DEFAULT_RUNS = [(192, 1, 5, True, 130, 0.0), (128, 1, -1, False, 90, 0.0), (96, 3, 4, True, 80, 0.2),
+                 (64, 1, 0, True, 40, 0.0), (48, 2, 7, True, 60, 0.1)]
+# the RadSearch knobs the runs above leave at their defaults: count_law = 1 (inverse square), bbox / observation_area
+# (offset origin with negative coordinates, a 1720 x 1720 arena just above the 1000 max-distance floor, arenas spanning
+# +-16000 and +-16383), k_max above the obstruction count, and single-agent runs through the tile program
+_KNOB_RUNS = {
+    "count_law1": ((128, 1, 5, True, 100, 0.0), dict(count_law=1)),
+    "offset_bbox": ((128, 1, 5, True, 100, 0.0), dict(bbox=(300, -200, 3300, 2900), obs_area=(150, 450))),
+    "offset_bbox_free": ((128, 1, 5, False, 100, 0.0), dict(bbox=(300, -200, 3300, 2900), obs_area=(150, 450))),
+    "offset_bbox_a3_count_law1": ((96, 3, 4, True, 80, 0.1), dict(bbox=(300, -200, 3300, 2900), obs_area=(150, 450),
+                                                                   count_law=1)),
+    "offset_bbox_tiled": ((128, 1, 3, True, 80, 0.0), dict(bbox=(300, -200, 3300, 2900), obs_area=(150, 450), tiled=True)),
+    "tight_1720": ((64, 1, 7, True, 60, 0.0), dict(bbox=(0, 0, 1720, 1720))),
+    "tight_1720_a2": ((64, 2, 7, True, 40, 0.1), dict(bbox=(0, 0, 1720, 1720))),
+    "large_16000": ((64, 1, 5, True, 60, 0.0), dict(bbox=(-16000, -16000, 16000, 16000))),
+    "large_16383": ((64, 1, 5, True, 60, 0.0), dict(bbox=(-16383, -16383, 16383, 16383))),
+    "kmax8": ((128, 1, -1, True, 80, 0.0), dict(k_max=8)),
+}
+
+
+@pytest.mark.parametrize("n,A,oc,enforce,T,idle,knobs",
+                         [pytest.param(*r, {}, id="-".join(str(x) for x in r)) for r in _DEFAULT_RUNS] +
+                         [pytest.param(*r, kw, id=name) for name, (r, kw) in _KNOB_RUNS.items()])
+def test_emulated_kernels_match_oracle_rollout(n, A, oc, enforce, T, idle, knobs):
     seed = 1000 + n
-    cfg = make_config(n_agents=A, obstruction_count=oc, enforce=enforce)
-    ob = co.OracleBatch(n, co.default_config(n_agents=A, obstruction_count=oc, enforce=int(enforce)), seed=seed, env_id0=7)
-    em = EmuEnv(n, cfg, seed=seed, env_id0=7)
+    knobs = dict(knobs)
+    tiled = knobs.pop("tiled", False)
+    geo = dict(bbox=knobs.get("bbox", (0, 0, 2700, 2700)), obs_area=knobs.get("obs_area", (200, 500)),
+               count_law=knobs.get("count_law", 0))
+    cfg = make_config(n_agents=A, obstruction_count=oc, enforce=enforce, k_max=knobs.get("k_max"), **geo)
+    ob = co.OracleBatch(n, co.default_config(n_agents=A, obstruction_count=oc, enforce=int(enforce), **geo), seed=seed,
+                        env_id0=7)
+    em = EmuEnv(n, cfg, seed=seed, env_id0=7, tiled=tiled)
     em.reset(0, flags=L.F_NEW_OBSTACLES)
     ob.reset()
     compare_state(em, ob, A)
