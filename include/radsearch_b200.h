@@ -324,6 +324,35 @@ int rs_maps_replay(const RsMapsConfig *cfg, const RsMapsState *st, const float *
 int rs_sizeof_maps_config(void);
 int rs_sizeof_maps_state(void);
 
+/* ---- fused GRU actor-critic inference (the RAD-A2C core, algos/test_environment/core.py) ----------------------------
+ * torch.nn.GRUCell(d_in, hidden) -> policy head over the 8 moves and value head, one thread per row m of the batch (env-
+ * major n*A + a for multi-agent batches), float32 throughout (no tensor cores).  params: the packed weights in torch's
+ * row-major order, weight_ih [3H][d_in] | weight_hh [3H][H] | bias_ih | bias_hh | policy head (W1, b1, W2, b2, or W, b)
+ * | value head (the same), rs_policy_param_count floats.  obs [rows][11], pred [rows][2] (the last two input columns, only
+ * with d_in = 13, NULL otherwise), hidden [rows][H]. */
+typedef struct RsPolicyConfig {
+    int32_t d_in;                /* 11, or 13 (obs + a caller-supplied source prediction)                         */
+    int32_t hidden;              /* H, 1..64                                                                      */
+    int32_t pi_hidden;           /* 0 = Linear(H, 8); P in 1..64 = Linear(H, P), activation, Linear(P, 8)          */
+    int32_t v_hidden;            /* 0 = Linear(H, 1); V in 1..64 = Linear(H, V), activation, Linear(V, 1)          */
+    int32_t activation;          /* 0 tanh, 1 relu (both heads)                                                   */
+} RsPolicyConfig;
+/* floats in the packed buffer; < 0 for a config outside the ranges above */
+int rs_policy_param_count(const RsPolicyConfig *cfg);
+/* hidden <- GRUCell(x, hidden) in place (torch's gate order r, z, n; h' = n + z (h - n)); value = value head of h';
+ * logp = log_softmax of the policy head at the sampled action; action (int32) = the first index of the maximum of
+ * logp_k + g_k, g_k = -log(-log u_k), u_k = ((x_k >> 8) + 0.5) 2^-24 for the 8 words x_k of Philox4x32-10 with key seed
+ * and counters (row_id0 + m, 4<<24 | b, *ctr lo, *ctr hi), b = 0, 1.  ctr: device uint64, read by every CTA and advanced
+ * by one by the last CTA to finish (ticket: device uint32, zero between launches), so a captured call draws fresh noise
+ * on every replay.  row_id0 + rows <= 2^32: the global row id makes the actions independent of how rows shard. */
+int rs_policy_act(const RsPolicyConfig *cfg, const float *params, const float *obs, const float *pred, float *hidden,
+                  int32_t *action, float *value, float *logp, int rows, uint32_t row_id0, uint64_t seed, uint64_t *ctr,
+                  uint32_t *ticket, void *stream);
+/* value = value head of GRUCell(x, hidden), hidden not written: the bootstrap value of the next observation (T:462-487). */
+int rs_policy_value(const RsPolicyConfig *cfg, const float *params, const float *obs, const float *pred,
+                    const float *hidden, float *value, int rows, void *stream);
+int rs_sizeof_policy_config(void);
+
 const char *rs_last_error(void);
 int rs_version(void);
 /* sizeof checks for the binding */

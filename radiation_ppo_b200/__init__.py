@@ -15,8 +15,9 @@ from .evaluate import (MonteCarloEvaluator, MonteCarloResults, TeamEvalPolicy, T
                        uniform_policy)
 from .rollout_stats import EpisodeStats
 from .rollout import RolloutCollector, TeamRolloutCollector, TeamRolloutPolicy
+from .policy import FusedGruPolicy
 
 __all__ = ["RadSearch", "StepResult", "HostStepBuffers", "PPOBuffer", "BatchedPPOBuffer", "gae_advantages", "advantage_statistics",
            "normalize_advantages_", "combined_shape", "shard_range", "BatchedMapsBuffer", "MapsBuffer", "MonteCarloEvaluator", "MonteCarloResults", "TeamMonteCarloResults",
            "TeamEvalPolicy", "uniform_policy", "EpisodeStats", "RolloutCollector",
-           "TeamRolloutCollector", "TeamRolloutPolicy", "episode_ranges", "RadSearchLibraryError", "_lib"]
+           "TeamRolloutCollector", "TeamRolloutPolicy", "FusedGruPolicy", "episode_ranges", "RadSearchLibraryError", "_lib"]

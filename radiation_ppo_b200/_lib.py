@@ -21,7 +21,8 @@ EXPORTS = [
     "rs_step", "rs_reset", "rs_prepare", "rs_bump_ctr", "rs_load_scenarios", "rs_query_shortest_path", "rs_gae", "rs_adv_stats", "rs_adv_normalize", "rs_last_error",
     "rs_version", "rs_sizeof_config", "rs_sizeof_state", "rs_maps_update", "rs_maps_reset", "rs_sizeof_maps_config",
     "rs_sizeof_maps_state", "rs_pack_rollout", "rs_episode_table", "rs_rollout_pre", "rs_rollout_post",
-    "rs_rollout_pre_team", "rs_rollout_post_team", "rs_maps_replay", "rs_eval_step",
+    "rs_rollout_pre_team", "rs_rollout_post_team", "rs_maps_replay", "rs_eval_step", "rs_policy_param_count",
+    "rs_policy_act", "rs_policy_value", "rs_sizeof_policy_config",
 ]
 MS_CELL_RANGE, MS_LOG_FULL, MS_PRED_RANGE = 1, 2, 4
 MR_BAD_RANGE = 8
@@ -65,6 +66,10 @@ class RsMapsState(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in (
         "actor", "critic", "log_cell", "log_val", "log_len", "last_cell", "last_pred", "std", "std_count",
         "visit_lut", "status")]
+
+
+class RsPolicyConfig(C.Structure):
+    _fields_ = [(n, C.c_int32) for n in ("d_in", "hidden", "pi_hidden", "v_hidden", "activation")]
 
 
 class RadSearchLibraryError(RuntimeError):
@@ -125,6 +130,14 @@ def declare(lib, prefix="rs_"):
         lib.rs_maps_replay.argtypes = [mcp, msp, vp, vp, vp, i32, i32, vp, i32, vp, vp, vp, vp, vp]
         lib.rs_eval_step.restype = i32
         lib.rs_eval_step.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, f64, vp, vp, vp, i32, i32, i32, vp]
+        pcp = C.POINTER(RsPolicyConfig)
+        lib.rs_policy_param_count.restype = i32
+        lib.rs_policy_param_count.argtypes = [pcp]
+        lib.rs_policy_act.restype = i32
+        lib.rs_policy_act.argtypes = [pcp, vp, vp, vp, vp, vp, vp, vp, i32, u32, u64, vp, vp, vp]
+        lib.rs_policy_value.restype = i32
+        lib.rs_policy_value.argtypes = [pcp, vp, vp, vp, vp, vp, i32, vp]
+        lib.rs_sizeof_policy_config.restype = i32
         lib.rs_sizeof_maps_config.restype = i32
         lib.rs_sizeof_maps_state.restype = i32
         lib.rs_last_error.restype = C.c_char_p
@@ -147,7 +160,8 @@ def load():
             raise RadSearchLibraryError(f"{LIB_PATH} lacks symbols {missing}")
         declare(lib)
         if lib.rs_sizeof_config() != C.sizeof(RsConfig) or lib.rs_sizeof_state() != C.sizeof(RsState) or \
-                lib.rs_sizeof_maps_config() != C.sizeof(RsMapsConfig) or lib.rs_sizeof_maps_state() != C.sizeof(RsMapsState):
+                lib.rs_sizeof_maps_config() != C.sizeof(RsMapsConfig) or lib.rs_sizeof_maps_state() != C.sizeof(RsMapsState) or \
+                lib.rs_sizeof_policy_config() != C.sizeof(RsPolicyConfig):
             raise RadSearchLibraryError("struct layout mismatch between _lib.py and libradsearch_b200.so")
         _lib = lib
     return _lib
