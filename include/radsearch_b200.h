@@ -353,6 +353,27 @@ int rs_policy_value(const RsPolicyConfig *cfg, const float *params, const float 
                     const float *hidden, float *value, int rows, void *stream);
 int rs_sizeof_policy_config(void);
 
+/* ---- PPO loss and gradient of the same actor-critic (the update's forward and backpropagation through time) --------
+ * One launch: the clipped PPO loss of M columns x T steps of a BatchedPPOBuffer, in its own [T][N] layout, and its exact
+ * gradient with respect to every packed parameter.  obs [T][N][11], pred [T][N][2] (d_in = 13 only), act [T][N] (float
+ * action indices), adv [T][N] (normalised), ret, logp [T][N], end [T][N] (uint8 path ends).  columns: int32 [M], the
+ * buffer columns of the minibatch (NULL: all of them, M = N).  Column m starts from h = 0 at t = 0 and step t reads
+ * h_{t-1} (1 - end[t-1]), the restart rule of rs_rollout_post.  With c = 1 / (T M), rho = exp(logp(a) - logp_old) and
+ * eps = clip_ratio,
+ *     L = w_pi c sum -min(rho A, clamp(rho, 1 - eps, 1 + eps) A) + w_v c sum (v - ret)^2
+ * and grad (rs_policy_param_count floats, overwritten) = dL/dparams with torch autograd's conventions (minimum splits a
+ * tie evenly, clamp passes the gradient on the closed interval).  stats (8 doubles, [0..5] written): sum -min(...),
+ * sum (v - ret)^2, sum (logp_old - logp), sum of the policy's entropy, rows with |rho - 1| > eps, and rows skipped (a
+ * column index outside 0..N-1 skips its T rows; an action outside 0..7 its row; skipped rows add nothing).  workspace:
+ * rs_policy_grad_workspace_bytes, device memory (the hidden states of every step, [T][M][H] floats, and per-CTA
+ * partials); ticket: device uint32, zero between launches.  No host synchronisation; CUDA-graph capturable; the result
+ * is bit-identical from call to call. */
+int64_t rs_policy_grad_workspace_bytes(const RsPolicyConfig *cfg, int32_t T, int32_t M);
+int rs_policy_ppo_grad(const RsPolicyConfig *cfg, const float *params, const float *obs, const float *pred, const float *act,
+                       const float *adv, const float *ret, const float *logp, const uint8_t *end, const int32_t *columns,
+                       int32_t T, int32_t N, int32_t M, double clip_ratio, double w_pi, double w_v, float *grad,
+                       double *stats, void *workspace, uint32_t *ticket, void *stream);
+
 const char *rs_last_error(void);
 int rs_version(void);
 /* sizeof checks for the binding */

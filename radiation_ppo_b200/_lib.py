@@ -22,7 +22,7 @@ EXPORTS = [
     "rs_version", "rs_sizeof_config", "rs_sizeof_state", "rs_maps_update", "rs_maps_reset", "rs_sizeof_maps_config",
     "rs_sizeof_maps_state", "rs_pack_rollout", "rs_episode_table", "rs_rollout_pre", "rs_rollout_post",
     "rs_rollout_pre_team", "rs_rollout_post_team", "rs_maps_replay", "rs_eval_step", "rs_policy_param_count",
-    "rs_policy_act", "rs_policy_value", "rs_sizeof_policy_config",
+    "rs_policy_act", "rs_policy_value", "rs_sizeof_policy_config", "rs_policy_grad_workspace_bytes", "rs_policy_ppo_grad",
 ]
 MS_CELL_RANGE, MS_LOG_FULL, MS_PRED_RANGE = 1, 2, 4
 MR_BAD_RANGE = 8
@@ -138,6 +138,11 @@ def declare(lib, prefix="rs_"):
         lib.rs_policy_value.restype = i32
         lib.rs_policy_value.argtypes = [pcp, vp, vp, vp, vp, vp, i32, vp]
         lib.rs_sizeof_policy_config.restype = i32
+        lib.rs_policy_grad_workspace_bytes.restype = i64
+        lib.rs_policy_grad_workspace_bytes.argtypes = [pcp, i32, i32]
+        lib.rs_policy_ppo_grad.restype = i32
+        lib.rs_policy_ppo_grad.argtypes = [pcp, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, f64, f64, f64, vp, vp, vp, vp,
+                                           vp]
         lib.rs_sizeof_maps_config.restype = i32
         lib.rs_sizeof_maps_state.restype = i32
         lib.rs_last_error.restype = C.c_char_p

@@ -13,11 +13,14 @@ Supported modules (anything else raises ValueError):
   value head   Linear(H, 1), or Sequential(Linear(H, V), activation, Linear(V, 1)); both heads use the same activation
 All parameters float32.  The arithmetic is float32 FMAs (no TF32), so the log-probabilities the collector stores match the
 ones the torch modules recompute in the PPO ratio to float32 rounding.
+
+`loss_and_grad` is the other half of the epoch: the PPO loss of a minibatch of a BatchedPPOBuffer's columns and its
+gradient by backpropagation through time, in one launch (rs_policy_ppo_grad), accumulated into the modules' .grad.
 """
 from __future__ import annotations
 
 import ctypes as C
-from typing import List, Optional, Tuple
+from typing import Dict, List, Optional, Tuple
 
 import torch
 
@@ -72,6 +75,7 @@ class FusedGruPolicy:
     hidden_state: float32 [num_rows, H], contiguous, restarted in place by rs_rollout_post.
     policy(obs, t) -> actions: MonteCarloEvaluator.run's policy; t == 0 restarts every row.
     sync(): repack the weights from the modules (after an optimiser step), on the current stream.
+    loss_and_grad(buf, ...): PPO loss and gradient of a buffer's columns into the modules' .grad (see there).
     Everything is queued on the current stream without a host synchronisation; the call counter lives on the device, so
     a captured act() draws fresh noise on every replay."""
 
@@ -122,6 +126,10 @@ class FusedGruPolicy:
         self.v_next = torch.zeros(num_rows, dtype=torch.float32, device=dev)
         self.ctr = torch.zeros(1, dtype=torch.int64, device=dev)        # call counter of the action noise (uint64 on the device)
         self.ticket = torch.zeros(1, dtype=torch.int32, device=dev)     # CTA completion counter, zero between launches
+        self.grad_ticket = torch.zeros(1, dtype=torch.int32, device=dev)  # the same, for rs_policy_ppo_grad
+        self._grad = torch.empty(count, dtype=torch.float32, device=dev)
+        self._stats = torch.zeros(8, dtype=torch.float64, device=dev)
+        self._workspace = {}                                             # (T, M) -> uint8 device buffer
         self._lib = lib
         self._fixed = [C.c_void_p(t.data_ptr()) for t in (self.params, self.h, self.action, self.val, self.logp, self.v_next,
                                                            self.ctr, self.ticket)]
@@ -178,3 +186,76 @@ class FusedGruPolicy:
         if t == 0:
             self.reset_state(None)
         return self.act(obs)[0]
+
+    def loss_and_grad(self, buf, pred: Optional[torch.Tensor] = None, columns: Optional[torch.Tensor] = None,
+                      clip_ratio: float = 0.2, w_pi: float = 1.0, w_v: float = 0.5) -> Dict[str, torch.Tensor]:
+        """PPO loss of M columns x T steps of `buf` (a BatchedPPOBuffer after get(): advantages normalised) and its exact
+        gradient with respect to the modules' parameters, one rs_policy_ppo_grad launch on the current stream with no host
+        synchronisation (CUDA-graph capturable once the workspace of (T, M) exists).  With c = 1 / (T M), rho =
+        exp(logp(a) - logp_old):
+
+            L = w_pi c sum -min(rho A, clamp(rho, 1 - clip_ratio, 1 + clip_ratio) A) + w_v c sum (v - ret)^2
+
+        w_pi = 1, w_v = 0.5 is bench.py's update; w_pi = 0 or w_v = 0 gives one head's gradient alone (separate optimisers).
+        The gradient is accumulated into each parameter's .grad (set where None), as loss.backward() would.
+
+        pred: [T, N, 2] for a 13-wide trunk (the source predictions the policy read).  columns: int32 [M] buffer columns of
+        the minibatch (default all N; a team buffer's agent a is columns n * A + a).  Column m restarts from h = 0 at t = 0
+        and after every path end (the rule of the collection loop), so the first steps of a column whose episode began in
+        the previous epoch see a different state than when they were sampled: their ratio is not exactly 1 even before an
+        optimiser step.  The weights are repacked first (sync()), so the current parameters are differentiated.
+
+        Returns 0-d device tensors: loss (= L), loss_pi and loss_v (the two means, unweighted), approx_kl (mean logp_old -
+        logp), entropy (mean), clip_frac (mean |rho - 1| > clip_ratio), over the rows that count, and skipped (rows left
+        out because the column index is outside 0..N-1 or the action outside 0..7)."""
+        T, N = buf.T, buf.N
+        if (pred is None) != (self.d_in == 11):
+            raise ValueError("a 13-wide policy needs pred [T, N, 2]; an 11-wide one takes none")
+        dev = self.device
+        if pred is not None:
+            pred = self._rows(pred, T * N * 2, "pred")
+        if columns is None:
+            M = N
+        else:
+            columns = columns.to(device=dev, dtype=torch.int32).contiguous().view(-1)
+            M = columns.numel()
+            if M < 1:
+                raise ValueError("columns is empty")
+        ws = self._workspace.get((T, M))
+        if ws is None:
+            nbytes = self._lib.rs_policy_grad_workspace_bytes(C.byref(self.cfg), T, M)
+            L.check(0 if nbytes >= 0 else int(nbytes), "rs_policy_grad_workspace_bytes")
+            ws = self._workspace[(T, M)] = torch.empty(int(nbytes), dtype=torch.uint8, device=dev)
+        self.sync()
+        rows = [self._rows(x, T * N, name) for x, name in ((buf.act_buf, "act"), (buf.adv_buf, "adv"), (buf.ret_buf, "ret"),
+                                                            (buf.logp_buf, "logp"))]
+        obs = self._rows(buf.obs_buf, T * N * L.OBS_DIM, "obs")
+        end = buf.end_buf
+        if end.dtype != torch.uint8 or not end.is_contiguous() or end.device != dev:
+            raise ValueError("buf.end_buf must be a contiguous uint8 tensor on the policy's device")
+        L.check(self._lib.rs_policy_ppo_grad(C.byref(self.cfg), _ptr(self.params), _ptr(obs), _ptr(pred), *map(_ptr, rows),
+                                             _ptr(end), _ptr(columns), T, N, M, float(clip_ratio), float(w_pi), float(w_v),
+                                             _ptr(self._grad), _ptr(self._stats), _ptr(ws), _ptr(self.grad_ticket),
+                                             self._stream()), "rs_policy_ppo_grad")
+        with torch.no_grad():
+            off = 0
+            for prm in self._params:
+                g = self._grad[off:off + prm.numel()].view_as(prm)
+                off += prm.numel()
+                if prm.grad is None:
+                    prm.grad = g.clone()
+                else:
+                    prm.grad.add_(g)
+        st = self._stats
+        c = 1.0 / (T * M)
+        counted = (T * M - st[5]).clamp(min=1.0)
+        loss_pi, loss_v = st[0] * c, st[1] * c
+        return dict(loss=w_pi * loss_pi + w_v * loss_v, loss_pi=loss_pi, loss_v=loss_v, approx_kl=st[2] / counted,
+                    entropy=st[3] / counted, clip_frac=st[4] / counted, skipped=st[5])
+
+    def _rows(self, x: torch.Tensor, numel: int, what: str) -> torch.Tensor:
+        if x.dtype != torch.float32 or not x.is_contiguous() or x.device != self.device:
+            x = x.to(device=self.device, dtype=torch.float32).contiguous()
+        if x.numel() != numel:
+            raise ValueError(f"{what} must hold {numel} floats, got shape {tuple(x.shape)}")
+        return x
