@@ -205,7 +205,7 @@ class FusedGruPolicy:
         the previous epoch see a different state than when they were sampled: their ratio is not exactly 1 even before an
         optimiser step.  The weights are repacked first (sync()), so the current parameters are differentiated.
 
-        Returns 0-d device tensors: loss (= L), loss_pi and loss_v (the two means, unweighted), approx_kl (mean logp_old -
+        Returns fresh 0-d device tensors, which a later call does not overwrite: loss (= L), loss_pi and loss_v (the two means, unweighted), approx_kl (mean logp_old -
         logp), entropy (mean), clip_frac (mean |rho - 1| > clip_ratio), over the rows that count, and skipped (rows left
         out because the column index is outside 0..N-1 or the action outside 0..7)."""
         T, N = buf.T, buf.N
@@ -251,7 +251,7 @@ class FusedGruPolicy:
         counted = (T * M - st[5]).clamp(min=1.0)
         loss_pi, loss_v = st[0] * c, st[1] * c
         return dict(loss=w_pi * loss_pi + w_v * loss_v, loss_pi=loss_pi, loss_v=loss_v, approx_kl=st[2] / counted,
-                    entropy=st[3] / counted, clip_frac=st[4] / counted, skipped=st[5])
+                    entropy=st[3] / counted, clip_frac=st[4] / counted, skipped=st[5].clone())
 
     def _rows(self, x: torch.Tensor, numel: int, what: str) -> torch.Tensor:
         if x.dtype != torch.float32 or not x.is_contiguous() or x.device != self.device:
