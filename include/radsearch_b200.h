@@ -20,6 +20,8 @@
  *                                  RADTEAM_core.py:188-277) in the call order of train.py:305-311, 333-341, 436, 469, 509, 548;
  *                                  mode 2 = StatBuff (algos/test_environment/core.py:55-79) + clip to [-8, 8]
  *                                  (algos/test_environment/ppo.py:502, 518)
+ *   rs_pfgru_predict / _peek / _restart   PFGRUCell.forward of the RAD-A2C source localiser
+ *                                  (RADA2C_core.py:215-307) and init_hidden, for T:326, 345-353, 470-477, 509-511
  */
 #ifndef RADSEARCH_B200_H
 #define RADSEARCH_B200_H
@@ -373,6 +375,51 @@ int rs_policy_ppo_grad(const RsPolicyConfig *cfg, const float *params, const flo
                        const float *adv, const float *ret, const float *logp, const uint8_t *end, const int32_t *columns,
                        int32_t T, int32_t N, int32_t M, double clip_ratio, double w_pi, double w_v, float *grad,
                        double *stats, void *workspace, uint32_t *ticket, void *stream);
+
+/* ---- fused PFGRU source localiser inference (the particle-filter GRU of RAD-A2C, RADA2C_core.py:215-307) -----------
+ * One warp per row m of the batch (env-major n*A + a), float32 throughout (no tensor cores).  State: particles
+ * [rows][K][H] and log_weights [rows][K], float32.  x = obs[m][0 .. d_in) (obs [rows][11]).  One step, with [a | b] the
+ * concatenation hidden part first:
+ *   z = sigmoid(fc_z[h0 | x]), r = sigmoid(fc_r[h0 | x]), (mu, nu) = fc_n[r h0 | x] (first H outputs mu, next H nu),
+ *   n = tanh(mu + eps softplus(nu)), eps ~ N(0, 1) per element, h1 = (1 - z) n + z h0,
+ *   p1 = log_softmax(fc_obs[h1 | x] + p0) over the K particles;
+ *   resample = 1: q = alpha exp(p1) + (1 - alpha) / K, i_k = the first i with u_k C_{K-1} < C_i (C the prefix sum of q in
+ *   particle order), h_k = h1[i_k], p_k = p1[i_k] - log(alpha w + (1 - alpha) / K), w = exp(p1[i_k]), p -= logsumexp(p);
+ *   resample = 0: h = h1, p = p1;
+ *   pred = hid_obs(sum_k exp(p_k) h_k), hid_obs = Linear(H, W) -> ReLU -> Linear(W, 2).
+ * params: fc_z.weight, fc_z.bias, fc_r.*, fc_n.*, fc_obs.*, hid_obs[0].*, hid_obs[2].*, torch row-major,
+ * rs_pfgru_param_count floats.
+ * Noise: Philox4x32-10 with key seed and counter (row_id0 + m, 5<<24 | block, *ctr lo, *ctr hi); every word x gives the
+ * uniform ((x >> 8) + 0.5) 2^-24.  Blocks: predict eps of particle k, elements 4g..4g+3: k*16 + g (Box-Muller: eps_4g =
+ * sqrt(-2 ln u0) cos 2pi u1, eps_4g+1 = sqrt(-2 ln u0) sin 2pi u1, eps_4g+2/3 the same of u2, u3); predict u_k: 1024 + k/4,
+ * word k%4; peek: 2048 + the predict blocks; restart element j of particle k: 4096 + k*16 + j/4, word j%4.  ctr: device
+ * uint64, read by all three calls and advanced by one by the last CTA of a predict (ticket: device uint32, zero between
+ * launches), so a captured predict draws fresh noise on every replay.  row_id0 + rows <= 2^32: the global row id makes
+ * the results independent of how rows shard.  mask[rows] u8 (NULL = all rows): row m is selected when mask[m] &
+ * mask_bits != 0 (mask_bits 0 = any non-zero byte).  All calls are asynchronous and CUDA-graph capturable. */
+typedef struct RsPfgruConfig {
+    int32_t d_in;                /* input columns taken from the observation, 1..11 (the reference: 3)              */
+    int32_t hidden;              /* H, 1..64                                                                      */
+    int32_t particles;           /* K, 1..64                                                                      */
+    int32_t obs_hidden;          /* W, the hidden width of hid_obs, 1..64                                         */
+    int32_t resample;            /* 1: soft resampling after every step, 0: none                                  */
+    float alpha;                 /* soft-resampling alpha, (0, 1]                                                 */
+} RsPfgruConfig;
+/* floats in the packed buffer; < 0 for a config outside the ranges above */
+int rs_pfgru_param_count(const RsPfgruConfig *cfg);
+/* one step of every row: the state is replaced in place, pred_out [rows][2] written */
+int rs_pfgru_predict(const RsPfgruConfig *cfg, const float *params, const float *obs, float *particles, float *log_weights,
+                     float *pred_out, int32_t rows, uint32_t row_id0, uint64_t seed, uint64_t *ctr, uint32_t *ticket,
+                     void *stream);
+/* the same step on the current state of the selected rows, pred_out written for those rows only; the state and ctr are
+ * not written */
+int rs_pfgru_peek(const RsPfgruConfig *cfg, const float *params, const float *obs, const float *particles,
+                  const float *log_weights, float *pred_out, const uint8_t *mask, int32_t mask_bits, int32_t rows,
+                  uint32_t row_id0, uint64_t seed, const uint64_t *ctr, void *stream);
+/* restart of the selected rows: h ~ U[0, 1) per element, p = -log K */
+int rs_pfgru_restart(const RsPfgruConfig *cfg, float *particles, float *log_weights, const uint8_t *mask, int32_t mask_bits,
+                     int32_t rows, uint32_t row_id0, uint64_t seed, const uint64_t *ctr, void *stream);
+int rs_sizeof_pfgru_config(void);
 
 const char *rs_last_error(void);
 int rs_version(void);

@@ -23,6 +23,7 @@ EXPORTS = [
     "rs_sizeof_maps_state", "rs_pack_rollout", "rs_episode_table", "rs_rollout_pre", "rs_rollout_post",
     "rs_rollout_pre_team", "rs_rollout_post_team", "rs_maps_replay", "rs_eval_step", "rs_policy_param_count",
     "rs_policy_act", "rs_policy_value", "rs_sizeof_policy_config", "rs_policy_grad_workspace_bytes", "rs_policy_ppo_grad",
+    "rs_pfgru_param_count", "rs_pfgru_predict", "rs_pfgru_peek", "rs_pfgru_restart", "rs_sizeof_pfgru_config",
 ]
 MS_CELL_RANGE, MS_LOG_FULL, MS_PRED_RANGE = 1, 2, 4
 MR_BAD_RANGE = 8
@@ -70,6 +71,10 @@ class RsMapsState(C.Structure):
 
 class RsPolicyConfig(C.Structure):
     _fields_ = [(n, C.c_int32) for n in ("d_in", "hidden", "pi_hidden", "v_hidden", "activation")]
+
+
+class RsPfgruConfig(C.Structure):
+    _fields_ = [(n, C.c_int32) for n in ("d_in", "hidden", "particles", "obs_hidden", "resample")] + [("alpha", C.c_float)]
 
 
 class RadSearchLibraryError(RuntimeError):
@@ -143,6 +148,16 @@ def declare(lib, prefix="rs_"):
         lib.rs_policy_ppo_grad.restype = i32
         lib.rs_policy_ppo_grad.argtypes = [pcp, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, f64, f64, f64, vp, vp, vp, vp,
                                            vp]
+        fcp = C.POINTER(RsPfgruConfig)
+        lib.rs_pfgru_param_count.restype = i32
+        lib.rs_pfgru_param_count.argtypes = [fcp]
+        lib.rs_pfgru_predict.restype = i32
+        lib.rs_pfgru_predict.argtypes = [fcp, vp, vp, vp, vp, vp, i32, u32, u64, vp, vp, vp]
+        lib.rs_pfgru_peek.restype = i32
+        lib.rs_pfgru_peek.argtypes = [fcp, vp, vp, vp, vp, vp, vp, i32, i32, u32, u64, vp, vp]
+        lib.rs_pfgru_restart.restype = i32
+        lib.rs_pfgru_restart.argtypes = [fcp, vp, vp, vp, i32, i32, u32, u64, vp, vp]
+        lib.rs_sizeof_pfgru_config.restype = i32
         lib.rs_sizeof_maps_config.restype = i32
         lib.rs_sizeof_maps_state.restype = i32
         lib.rs_last_error.restype = C.c_char_p
@@ -166,7 +181,8 @@ def load():
         declare(lib)
         if lib.rs_sizeof_config() != C.sizeof(RsConfig) or lib.rs_sizeof_state() != C.sizeof(RsState) or \
                 lib.rs_sizeof_maps_config() != C.sizeof(RsMapsConfig) or lib.rs_sizeof_maps_state() != C.sizeof(RsMapsState) or \
-                lib.rs_sizeof_policy_config() != C.sizeof(RsPolicyConfig):
+                lib.rs_sizeof_policy_config() != C.sizeof(RsPolicyConfig) or \
+                lib.rs_sizeof_pfgru_config() != C.sizeof(RsPfgruConfig):
             raise RadSearchLibraryError("struct layout mismatch between _lib.py and libradsearch_b200.so")
         _lib = lib
     return _lib

@@ -14,7 +14,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 SRC_DIR = os.path.join(HERE, "csrc")
 OUT_DIR = os.path.join(HERE, "_C")
 LIB = os.path.join(OUT_DIR, "libradsearch_b200.so")
-SOURCES = ["rs_kernels.cu", "rs_gae.cu", "rs_maps.cu", "rs_pack.cu", "rs_rollout.cu", "rs_eval.cu", "rs_policy.cu", "rs_policy_grad.cu"]
+SOURCES = ["rs_kernels.cu", "rs_gae.cu", "rs_maps.cu", "rs_pack.cu", "rs_rollout.cu", "rs_eval.cu", "rs_policy.cu", "rs_policy_grad.cu",
+           "rs_pfgru.cu"]
 NVCC_FLAGS = [
     "-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-fmad=false",
     "-Xcompiler", "-fPIC", "-shared", "-cudart", "static",

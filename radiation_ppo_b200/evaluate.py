@@ -135,7 +135,10 @@ class MonteCarloEvaluator:
         self.intensity = torch.as_tensor(np.asarray(scenarios["intensity"]), dtype=torch.int32, device=self.env.device)
         self.background = torch.as_tensor(np.asarray(scenarios["bkg"]), dtype=torch.int32, device=self.env.device)
 
-    def run(self, policy: Policy, on_step: Optional[Callable[[int, torch.Tensor, torch.Tensor], None]] = None) -> MonteCarloResults:
+    def run(self, policy: Policy, on_step: Optional[Callable[[int, torch.Tensor, torch.Tensor], None]] = None,
+            localizer: Optional[Callable[[torch.Tensor, int], torch.Tensor]] = None) -> MonteCarloResults:
+        """Plays every scenario x run: actions = policy(obs, t), or with a localizer (e.g. pfgru.FusedPFGRU over the N*A
+        rows) policy(obs, t, localizer(obs, t)), the source prediction [N*A, 2] of a 13-wide policy."""
         env, S, R, A = self.env, self.n_scenarios, self.runs, self.env.number_agents
         N = S * R
         dev = env.device
@@ -147,7 +150,8 @@ class MonteCarloEvaluator:
         length = torch.zeros(N, dtype=torch.int32, device=dev)
         ret = torch.zeros(N, dtype=torch.float64, device=dev)
         for t in range(self.steps_per_episode):
-            acts = policy(obs, t).to(device=dev, dtype=torch.int32).reshape(N, A)
+            acts = policy(obs, t) if localizer is None else policy(obs, t, localizer(obs, t))
+            acts = acts.to(device=dev, dtype=torch.int32).reshape(N, A)
             obs, reward, team, done, _, _ = env.step_batch(acts, auto_reset=False)
             r = team if self.team_mode != "individual" else reward[:, 0]      # E:402-409 (agent 0's tally is reported)
             ret += torch.where(active, r, torch.zeros_like(r)).double()

@@ -73,7 +73,7 @@ class FusedGruPolicy:
     act(obs, pred=None) -> (action int32, value f32, logp f32), persistent [num_rows] tensors; advances hidden_state.
     value(obs, pred=None) -> f32 [num_rows], the value under the current hidden state (hidden_state untouched).
     hidden_state: float32 [num_rows, H], contiguous, restarted in place by rs_rollout_post.
-    policy(obs, t) -> actions: MonteCarloEvaluator.run's policy; t == 0 restarts every row.
+    policy(obs, t, pred=None) -> actions: MonteCarloEvaluator.run's policy; t == 0 restarts every row.
     sync(): repack the weights from the modules (after an optimiser step), on the current stream.
     loss_and_grad(buf, ...): PPO loss and gradient of a buffer's columns into the modules' .grad (see there).
     Everything is queued on the current stream without a host synchronisation; the call counter lives on the device, so
@@ -182,10 +182,10 @@ class FusedGruPolicy:
         else:
             self.h.masked_fill_(mask.reshape(-1, 1).to(device=self.device, dtype=torch.bool), 0.0)
 
-    def __call__(self, obs: torch.Tensor, t: int) -> torch.Tensor:
+    def __call__(self, obs: torch.Tensor, t: int, pred: Optional[torch.Tensor] = None) -> torch.Tensor:
         if t == 0:
             self.reset_state(None)
-        return self.act(obs)[0]
+        return self.act(obs, pred)[0]
 
     def loss_and_grad(self, buf, pred: Optional[torch.Tensor] = None, columns: Optional[torch.Tensor] = None,
                       clip_ratio: float = 0.2, w_pi: float = 1.0, w_v: float = 0.5) -> Dict[str, torch.Tensor]:

@@ -211,10 +211,13 @@ class BatchedPPOBuffer:
     ``agents=A`` (RAD-TEAM, TeamRolloutCollector): `num_columns` counts environments and the buffer has N*A env-major
     columns (column n*A + a, the memory order of the env's [N, A] outputs), plus `pred_buf` [T, N*A, 2], the PFGRU's
     source predictions the map observation was updated with (what BatchedMapsBuffer.replay needs besides the
-    observations and path ends).  GAE runs per column; agent_view() gives the [T, N] per-agent slices."""
+    observations and path ends).  GAE runs per column; agent_view() gives the [T, N] per-agent slices.
+
+    ``predictions=True`` gives a single-agent buffer `pred_buf` [T, N, 2] as well: the source predictions of a localiser
+    (pfgru.FusedPFGRU) that a 13-wide policy read, which its PPO ratio needs again (RolloutCollector(localizer=...))."""
 
     def __init__(self, observation_dimension: int, steps_per_epoch: int, num_columns: int, gamma: float = 0.99,
-                 lam: float = 0.90, device=None, agents: Optional[int] = None) -> None:
+                 lam: float = 0.90, device=None, agents: Optional[int] = None, predictions: bool = False) -> None:
         self.device = _need_cuda(device)
         L.load()
         if agents is not None and not 1 <= int(agents) <= L.MAX_A:
@@ -235,7 +238,7 @@ class BatchedPPOBuffer:
         self.boot_buf = z(T, N)
         self.end_buf = z(T, N, dt=torch.uint8)
         self.source_tar = z(T, N, 2)
-        self.pred_buf = None if self.A is None else torch.full((T, N, 2), float("nan"), dtype=torch.float32, device=self.device)
+        self.pred_buf = None if self.A is None and not predictions else torch.full((T, N, 2), float("nan"), dtype=torch.float32, device=self.device)
         self.stats = z(2, dt=torch.float64)
         self.ptr = 0
 
@@ -263,12 +266,15 @@ class BatchedPPOBuffer:
         return {"obs": self._obs_store[t + 1], "reward": self.rew_buf[t], "ended": self.end_buf[t]}
 
     def policy_rows(self, t: Optional[int] = None) -> Dict[str, torch.Tensor]:
-        """Rows of step t the policy side fills: obs (read), act / val / logp / boot / src (write)."""
+        """Rows of step t the policy side fills: obs (read), act / val / logp / boot / src (write), and pred (write) in a
+        buffer with predictions."""
         t = self.ptr if t is None else t
         rows = {"obs": self._obs_store[t], "act": self.act_buf[t], "val": self.val_buf[t], "logp": self.logp_buf[t],
                 "boot": self.boot_buf[t], "src": self.source_tar[t]}
         if self.A is not None:
             rows.update(pred=self.pred_buf[t], rew=self.rew_buf[t], end=self.end_buf[t])
+        elif self.pred_buf is not None:
+            rows.update(pred=self.pred_buf[t])
         return rows
 
     def agent_view(self, a: int) -> Dict[str, torch.Tensor]:

@@ -34,10 +34,11 @@ from .rollout_stats import EpisodeStats
 class RolloutPolicy(Protocol):
     def act(self, obs: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
         """obs [N, D] f32 -> (action int32 [N], state value f32 [N], log-probability f32 [N]); advances the policy's own
-        recurrent state (T:345-353)."""
+        recurrent state (T:345-353).  With a localizer the collector calls act(obs, pred), pred f32 [N, 2]."""
 
     def value(self, obs: torch.Tensor) -> torch.Tensor:
-        """State value f32 [N] of `obs` under the current recurrent state, without advancing it (T:470-477)."""
+        """State value f32 [N] of `obs` under the current recurrent state, without advancing it (T:470-477).  With a
+        localizer: value(obs, pred)."""
 
     def reset_state(self, mask: Optional[torch.Tensor]) -> None:
         """Restart the recurrent state of the envs in `mask` (bool [N]; None = all) (T:326, 509-511).  A policy that
@@ -53,10 +54,20 @@ class RolloutCollector:
     mode "graph" (needs an env with prefetch=True, use_cuda_graph=True): the env replays its captured step graph, whose
     outputs are the env's own fixed tensors, and the two bookkeeping launches that exist anyway carry them into the rows
     (49 bytes per env and step): fewer, cheaper launches per step when the host is the bottleneck.  A policy may read
-    `env.obs` and write `env.action_buffer` in place, so nothing else moves.  Both modes fill the buffer identically."""
+    `env.obs` and write `env.action_buffer` in place, so nothing else moves.  Both modes fill the buffer identically.
+
+    localizer (optional, e.g. pfgru.FusedPFGRU over the N rows; needs BatchedPPOBuffer(..., predictions=True)): the source
+    predictions of a 13-wide policy.  Per step t, in this order:
+      1. pred = localizer.predict(obs, out=buf.pred_buf[t])
+      2. action, value, logp = policy.act(obs, pred)
+      3. rs_rollout_pre, 4. the env step
+      5. v_next = policy.value(final_obs, localizer.peek(final_obs, mask=<the rows rs_rollout_post bootstraps>))
+      6. rs_rollout_post
+      7. localizer.reset_state(<ended rows>), the rows whose policy state rs_rollout_post restarts (not at the last step)
+    and localizer.reset_state(None) opens every epoch (T:326)."""
 
     def __init__(self, env: RadSearch, buf: BatchedPPOBuffer, policy: RolloutPolicy, stats: Optional[EpisodeStats] = None,
-                 mode: str = "rows"):
+                 mode: str = "rows", localizer=None):
         if env.number_agents != 1:
             raise ValueError("RolloutCollector drives single-agent envs (the RAD-A2C branch of train.py)")
         if not env.auto_reset:
@@ -67,7 +78,10 @@ class RolloutCollector:
             raise ValueError("mode must be 'rows' or 'graph'")
         if mode == "graph" and not env.use_cuda_graph:
             raise ValueError("mode='graph' needs an env created with prefetch=True, use_cuda_graph=True")
+        if localizer is not None and buf.pred_buf is None:
+            raise ValueError("a localizer needs a buffer with pred_buf (BatchedPPOBuffer(..., predictions=True))")
         self.env, self.buf, self.policy, self.stats, self.mode = env, buf, policy, stats, mode
+        self.localizer = localizer
         self._first = True
         # the rows of the (persistent) buffer every step writes: resolved once, not at every step
         self._rows = [buf.policy_rows(t) for t in range(buf.T)]
@@ -75,7 +89,7 @@ class RolloutCollector:
         self._outs_resolved = [env.resolve_outputs(o) for o in self._outs] if mode == "rows" else None
 
     def collect(self, gae_variant: int = 0) -> None:
-        env, buf, pol = self.env, self.buf, self.policy
+        env, buf, pol, loc = self.env, self.buf, self.policy, self.localizer
         T, N, D = buf.T, buf.N, buf.D
         lib = L.load()
         stream = C.c_void_p(torch.cuda.current_stream(env.device).cuda_stream)
@@ -89,6 +103,8 @@ class RolloutCollector:
             buf.ptr = 0
         self._first = False
         pol.reset_state(None)                                                        # T:326
+        if loc is not None:
+            loc.reset_state(None)
         hidden = getattr(pol, "hidden_state", None)                                  # [N, H] float32, restarted in place
         hdim = 0 if hidden is None else hidden.shape[1]
         st = [p(x) for x in (self.stats.fused_args() if self.stats is not None else (None,) * 5)]
@@ -99,7 +115,11 @@ class RolloutCollector:
         for t in range(T):
             rows, outs = self._rows[t], self._outs[t]
             last = t == T - 1
-            action, value, logp = pol.act(rows["obs"] if rows_mode else env_obs)
+            obs = rows["obs"] if rows_mode else env_obs
+            if loc is None:
+                action, value, logp = pol.act(obs)
+            else:
+                action, value, logp = pol.act(obs, loc.predict(obs, out=rows["pred"]))
             # row t of the buffer <- action, value, log-probability, source coordinates (T:416-428), one launch
             L.check(lib.rs_rollout_pre(p(action), p(value), p(logp), p_src, p(rows["act"]), p(rows["val"]), p(rows["logp"]),
                                        p(rows["src"]), None if rows_mode else p_obs, None if rows_mode else p(rows["obs"]), D, N,
@@ -111,11 +131,17 @@ class RolloutCollector:
                 env.step_batch(action, epoch_end=last)                               # captured graph, the env's own outputs
                 p_r, p_e, rr, er = p_rew, p_end, p(outs["reward"]), p(outs["ended"])
             # T:462-487 bootstrap where the trajectory was cut, T:509-511 recurrent state, T:361-391 episode statistics
-            v_next = pol.value(final_obs)
+            if loc is None:
+                v_next = pol.value(final_obs)
+            else:                           # the prediction for exactly the rows rs_rollout_post bootstraps below
+                ended = outs["ended"] if rows_mode else env.ended
+                v_next = pol.value(final_obs, loc.peek(final_obs, mask=None if last else ended, mask_bits=L.E_TIMEOUT))
             L.check(lib.rs_rollout_post(p_r, p_e, p_done, p_info, p(v_next), p(rows["boot"]), p_hidden, hdim, st[0], st[1],
                                         st[2], st[3], st[4], rr, er, N, int(last), stream), "rs_rollout_post")
             if hidden is None and not last:
                 pol.reset_state(outs["ended"] != 0)                                  # T:509-511
+            if loc is not None and not last:
+                loc.reset_state(outs["ended"])                                       # T:509-511 (ended byte != 0)
             buf.advance()
         buf.finish_paths(variant=gae_variant)
 
